@@ -15,7 +15,9 @@ the batch: init state -> consume all local rows -> (exchange) -> finalize -> pro
 `--impl reference` times only that CPU restatement (the reference runtime cannot be built here: no MPI).
 
 The line also carries `config.no_hint` (the same steps without the expected_groups hint, which the reference's API does not
-have; `--no-hint` makes that the headline run).  Other workloads, each printing the same kind of line:
+have; `--no-hint` makes that the headline run).  `--dump-outputs DIR` writes the result of the last timed step (float64
+DIR/<column>.npy, rows ordered by key) so that two builds can be compared array for array on the same seeded input.
+Other workloads, each printing the same kind of line:
   --workload join                           BASELINE.json configs[2], benchmarks/join_bench.py
   --workload shuffle                        raw-row variant of configs[3], benchmarks/shuffle_bench.py
   --aggs F1,F2.. [--nullable] [--key-dtype int32] [--val-dtype int32]
@@ -48,6 +50,7 @@ BYTES_PER_ROW = 16  # algorithmic bytes of the hash-aggregate scan (SURVEY.md §
 # shipping 2^27-row kernels): K1n 2.133 + 1.029 GB, K2n 1.116 + 0.000 GB = 4.279 GB = 31.9 B/row (16 read + 8 bucket write +
 # 8 bucket read by design).
 TRAFFIC_PER_ROW = {"spg": 3.220e9 / (1 << 26), "spgn": 4.279e9 / (1 << 27), "direct": 11.17e9 / (1 << 27)}
+DUMP_BYTES = 64 << 20  # --dump-outputs writes at most this much in all
 
 
 def parse_args():
@@ -77,7 +80,12 @@ def parse_args():
     ap.add_argument("--probe-batch", type=int, default=250_000_000)
     ap.add_argument("--sample-lo", type=int, default=1000, help="join parity: sorted row-set equality for keys in [lo, hi)")
     ap.add_argument("--sample-hi", type=int, default=1400)
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the result of the last timed step as float64 DIR/<column>.npy, "
+                    "rows ordered by key (default groupby workload, one process)")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    return args
 
 
 def peaks():
@@ -217,6 +225,25 @@ def reference_arm(args):
     print(json.dumps(line), flush=True)
 
 
+def write_outputs(out_dir, cols):
+    """--dump-outputs: the columns {name: device tensor} a caller of the timed path received, as DIR/<name>.npy in float64.
+    Rows are ordered by the first (key) column: the library's row order is not part of its result.  Above DUMP_BYTES in all,
+    a fixed seeded sample of the ordered rows is written, the same rows for the same arguments, so that the files of two builds
+    can be compared array for array."""
+    import numpy as np
+    import torch
+
+    names = list(cols)
+    order = torch.argsort(cols[names[0]])
+    cap = DUMP_BYTES // (8 * len(names))
+    if order.numel() > cap:
+        pick = np.sort(np.random.default_rng(0).choice(order.numel(), cap, replace=False))
+        order = order[torch.from_numpy(pick).to(order.device)]
+    os.makedirs(out_dir, exist_ok=True)
+    for name in names:
+        np.save(os.path.join(out_dir, f"{name}.npy"), cols[name][order].cpu().numpy().astype(np.float64))
+
+
 def workload_name(args):
     if args.gpus == 1:
         return f"{args.rows}-row int64 2-col, {args.groups}-group groupby SUM/COUNT on 1xB200 (BASELINE.json configs[1])"
@@ -226,6 +253,9 @@ def workload_name(args):
 
 def main():
     args = parse_args()
+    variant = args.aggs.replace(" ", "") != "sum,count" or args.nullable or args.key_dtype != "int64" or args.val_dtype != "int64"
+    if args.dump_outputs and (args.workload != "groupby" or args.impl != "b200" or variant):
+        sys.exit("--dump-outputs is implemented for the default groupby workload only")
     if args.workload == "join":
         from benchmarks import join_bench
 
@@ -239,7 +269,7 @@ def main():
     if args.impl == "reference":
         reference_arm(args)
         return
-    if args.aggs.replace(" ", "") != "sum,count" or args.nullable or args.key_dtype != "int64" or args.val_dtype != "int64":
+    if variant:
         from benchmarks import groupby_variant_bench
 
         groupby_variant_bench.run(args, ClockSampler, peaks)
@@ -258,6 +288,8 @@ def main():
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
     if world != args.gpus and world > 1:
         args.gpus = world
+    if args.dump_outputs and world > 1:
+        sys.exit("--dump-outputs writes the result of one process: run it with --gpus 1")
     _lib.require_gpu()
     torch.cuda.set_device(local_rank)
     dev = torch.device("cuda", local_rank)
@@ -280,7 +312,7 @@ def main():
 
     stats = {}
 
-    def one_step(tab, collect=False, profile=False, to_host=False, hint=None):
+    def one_step(tab, collect=False, profile=False, to_host=False, hint=None, keep=False):
         st = G.init_groupby_state(-1, (0,), ("sum", "count"), (0, 1, 2), (1, 1), parallel=world > 1,
                                   expected_groups=exp_groups_local if hint is None else hint,
                                   output_batch_size=1 << 40, device=local_rank, stream=stream_ptr)
@@ -294,6 +326,8 @@ def main():
         if to_host:
             res = [c.values_numpy(stream_ptr) for c in out.columns]
             stats["d2h"] = sum(a.nbytes for a in res)
+        if keep:  # the output columns are the state's memory: copy them before it is deleted
+            stats["kept"] = {nm: torch.as_tensor(c.data, device=dev)[:out.n_rows].clone() for nm, c in zip(out.names, out.columns)}
         if collect:
             cols = [torch.as_tensor(c.data, device=dev) for c in out.columns]
             stats["n_out"] = out.n_rows
@@ -358,12 +392,14 @@ def main():
     ev0, ev1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     barrier()
     ev0.record(stream)
-    for _ in range(args.steps):
-        one_step(table)
+    for i in range(args.steps):
+        one_step(table, keep=bool(args.dump_outputs) and i == args.steps - 1)
     ev1.record(stream)
     barrier()
     ms = ev0.elapsed_time(ev1)
     clocks = sampler.stop() if sampler else None
+    if args.dump_outputs:
+        write_outputs(args.dump_outputs, stats.pop("kept"))
 
     # the same steps WITHOUT the expected_groups hint (the reference's API has no such argument: a drop-in caller gets this
     # route — the state learns the cardinality from a 2^20-row prefix through the direct kernel, then takes the same kernels)

@@ -14,7 +14,6 @@ import numpy as np
 
 _HERE = os.path.dirname(os.path.abspath(__file__))
 _LIB = None
-_REF = None
 
 FT = {"size": 4, "sum": 6, "count": 7, "mean": 14, "min": 15, "max": 16}
 CT = {
@@ -73,27 +72,6 @@ def lib():
         L.oracle_synth_fill.argtypes = [C.c_void_p, C.c_void_p, C.c_int64, C.c_int64, C.c_int64, C.c_uint64]
         _LIB = L
     return _LIB
-
-
-def ref_lib():
-    """The reference's own vendored xxHash (oracle/_ref/libref_xxh3.so), or None if never built."""
-    global _REF
-    if _REF is None:
-        p = os.path.join(_HERE, "_ref", "libref_xxh3.so")
-        if not os.path.exists(p):
-            try:
-                build()
-            except Exception:
-                pass
-        if not os.path.exists(p):
-            return None
-        R = C.CDLL(p)
-        R.ref_hash_inner_32_i64.restype = C.c_uint32
-        R.ref_hash_inner_32_i64.argtypes = [C.c_int64, C.c_uint32]
-        R.ref_hash_inner_32_i32.restype = C.c_uint32
-        R.ref_hash_inner_32_i32.argtypes = [C.c_int32, C.c_uint32]
-        _REF = R
-    return _REF
 
 
 def _bitmap(valid):

@@ -1,6 +1,9 @@
 """GPU parity tests for the row->rank radix partition: placement identical to the reference's
 hash_to_rank(XXH3(key, SEED_HASH_PARTITION)) and bit-identical stable scatter versus the oracle."""
 
+import json
+import os
+
 import numpy as np
 import pandas as pd
 import pytest
@@ -13,6 +16,15 @@ from bodo_b200.table import CTable, Table
 from tests.helpers import table_to_device
 
 pytestmark = pytest.mark.gpu
+GOLDEN = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden")
+
+
+def _device_hash_to_rank(gpu_lib, keys, n_pes):
+    t = table_to_device(Table.from_pandas(pd.DataFrame({"k": keys})))
+    dest = torch.empty(len(keys), dtype=torch.int32, device="cuda")
+    ct = CTable(t)  # keep the cffi structs alive for the duration of the call
+    _lib.check(gpu_lib.b200_hash_to_rank(ct.ptr, n_pes, ffi.cast("int32_t*", dest.data_ptr()), ffi.NULL))
+    return dest.cpu().numpy()
 
 
 @pytest.mark.parametrize("n_pes", [1, 2, 3, 8, 64])
@@ -20,18 +32,18 @@ pytestmark = pytest.mark.gpu
 def test_hash_to_rank_matches_reference_placement(gpu_lib, oracle, n_pes, key_dtype):
     rng = np.random.default_rng(0)
     keys = rng.integers(np.iinfo(key_dtype).min, np.iinfo(key_dtype).max, 100_003).astype(key_dtype)
-    t = table_to_device(Table.from_pandas(pd.DataFrame({"k": keys})))
-    dest = torch.empty(len(keys), dtype=torch.int32, device="cuda")
-    ct = CTable(t)  # keep the cffi structs alive for the duration of the call
-    _lib.check(gpu_lib.b200_hash_to_rank(ct.ptr, n_pes, ffi.cast("int32_t*", dest.data_ptr()), ffi.NULL))
-    got = dest.cpu().numpy()
+    got = _device_hash_to_rank(gpu_lib, keys, n_pes)
     if key_dtype == np.int64:
         np.testing.assert_array_equal(got, oracle.hash_to_rank(keys, None, n_pes))
-    R = oracle.ref_lib()  # the reference's own vendored xxHash, when it was built in the authoring container
-    if R is not None:
-        f = R.ref_hash_inner_32_i64 if key_dtype == np.int64 else R.ref_hash_inner_32_i32
-        exp = np.array([f(int(k), 0xB0D01289) % n_pes for k in keys[:5000]])
-        np.testing.assert_array_equal(got[:5000], exp)
+    L = oracle.lib()
+    f = L.oracle_hash_inner_32_i64 if key_dtype == np.int64 else L.oracle_hash_inner_32_i32
+    np.testing.assert_array_equal(got[:5000], [f(int(k), oracle.SEED_HASH_PARTITION) % n_pes for k in keys[:5000]])
+    # the reference's own vendored xxHash: its known-answer vectors for the partition seed
+    width = "64" if key_dtype == np.int64 else "32"
+    vec = next(v for v in json.load(open(os.path.join(GOLDEN, "xxh3_hash_inner_32.json")))["vectors"]
+               if v["seed"] == oracle.SEED_HASH_PARTITION)
+    got = _device_hash_to_rank(gpu_lib, np.array(vec["keys" + width], dtype=key_dtype), n_pes)
+    np.testing.assert_array_equal(got, np.array(vec["hash" + width], dtype=np.uint64) % n_pes)
 
 
 @pytest.mark.parametrize("n_pes", [2, 8, 5])

@@ -70,16 +70,6 @@ def test_oracle_hash_matches_reference_known_answers(oracle):
             assert L.oracle_hash_inner_32_i32(k, seed) == h
 
 
-def test_oracle_hash_matches_reference_library_when_present(oracle):
-    R = oracle.ref_lib()
-    if R is None:
-        pytest.skip("oracle/_ref/libref_xxh3.so not built (no /root/reference here); known-answer vectors cover it")
-    L = oracle.lib()
-    rng = np.random.default_rng(1)
-    for k in rng.integers(-(2**63), 2**63 - 1, 5000):
-        assert L.oracle_hash_inner_32_i64(int(k), 0xB0D01289) == R.ref_hash_inner_32_i64(int(k), 0xB0D01289)
-
-
 def test_oracle_groupby_vs_pandas_random(oracle):
     rng = np.random.default_rng(0)
     n = 50_000
