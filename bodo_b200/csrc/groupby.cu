@@ -1003,11 +1003,7 @@ constexpr int SPG_MAX_OWNERS = 256;
 // K1 reserves one run per owner per tile with a global atomic on the owner's row counter: ~10^7 atomics per launch.  With
 // the 148 counters packed into ten cache lines K1's speed depended on where the array happened to land (0.80 ms against
 // 1.00 ms per 2^27 rows for the same SASS after an unrelated allocation moved it), so every counter gets its own line.
-#ifdef SPG_CNT_STRIDE_OVERRIDE  // scratch/spg_harness experiments only
-constexpr int SPG_CNT_STRIDE = SPG_CNT_STRIDE_OVERRIDE;
-#else
 constexpr int SPG_CNT_STRIDE = 16;
-#endif
 constexpr int SPG_STASH = 1024;     // K2: linear-probing stash slots for keys whose two buckets are full
 
 struct SpgArgs {
@@ -1033,13 +1029,9 @@ struct SpgArgs {
     int ns;                     // shared-memory table slots (K2)
     int n_pass;                 // K2 passes over each owner bucket (pass p keeps the keys of sub-range p): > 1 when the
                                 // estimated cardinality exceeds what the shared tables hold at once
+    int reserve_tickets;  // K2n flush: the global table is empty — a CTA reserves the group tickets of all its slots with one atomic
     const long long* hot_tab;   // [SPG_HOT_SLOTS] heavy-hitter keys found by spg_hot_sample_kernel (EMPTY_KEY = free), or null
     const int* n_hot;           // number of keys in hot_tab (device memory: K1 reads it, the host never waits for it)
-    // STATIC variant (experimental, B200_SPG_STATIC=1): every (owner, K1 CTA) pair has a private segment of bucket_cap rows
-    // inside the owner's bucket, so K1 needs no global run-reservation atomics; sub_cnt[owner * n_cta + cta] = rows written
-    unsigned int* sub_cnt;
-    int n_cta;
-    int reserve_tickets;  // K2n flush: the global table is empty — a CTA reserves the group tickets of all its slots with one atomic
 };
 
 // cheap in-kernel hash for owner / shared-table slot (placement inside one GPU is free to choose; the rank
@@ -1256,7 +1248,7 @@ __device__ __forceinline__ void tma_load_1d(void* smem_dst, const void* gsrc, ui
                  ::"r"(smem_u32(smem_dst)), "l"(gsrc), "r"(bytes), "r"(smem_u32(bar)) : "memory");
 }
 
-template <bool HAS_SUM, bool HAS_CNT, bool HOT = false, bool STATIC = false>
+template <bool HAS_SUM, bool HAS_CNT, bool HOT = false>
 __global__ void __launch_bounds__(SPG_TTHREADS, SPG_TCTAS) spg_partition_tma_kernel(const __grid_constant__ SpgArgs a) {
     extern __shared__ __align__(128) unsigned char smem_tma_raw[];  // own name: the other kernels declare smem_raw with 16-byte alignment
     long long* raw_k = (long long*)smem_tma_raw;                                   // [NB][SPG_TILE] keys
@@ -1283,11 +1275,6 @@ __global__ void __launch_bounds__(SPG_TTHREADS, SPG_TCTAS) spg_partition_tma_ker
         mbar_init(&mbar[1], 1);
         asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
     }
-    // STATIC: this CTA's private segment cursor per owner, and (cursor - local run start) for the copy-out
-    unsigned int* cursor = (unsigned int*)gbase;
-    unsigned int* cbase = cursor + SPG_MAX_OWNERS;
-    if (STATIC)
-        for (int j = tid; j < G; j += SPG_TTHREADS) cursor[j] = 0;
     for (int j = tid; j < G; j += SPG_TTHREADS) hist[j] = 0;
     __syncthreads();
     // full tiles come in through TMA; a trailing partial tile is loaded with ordinary loads
@@ -1357,7 +1344,7 @@ __global__ void __launch_bounds__(SPG_TTHREADS, SPG_TCTAS) spg_partition_tma_ker
         // reserve one run per owner: the global atomic's round trip (~1 us) is kept in a register and only waited for
         // after the staging pass, which needs the local prefix sums but not the global run start
         unsigned long long my_gbase = 0;
-        if (!STATIC && tid >= SPG_TTHREADS - G) { int ow = tid - (SPG_TTHREADS - G); unsigned int cnt = hist[ow]; if (cnt) my_gbase = atomicAdd(&a.bucket_cnt[ow * SPG_CNT_STRIDE], (unsigned long long)cnt); }
+        if (tid >= SPG_TTHREADS - G) { int ow = tid - (SPG_TTHREADS - G); unsigned int cnt = hist[ow]; if (cnt) my_gbase = atomicAdd(&a.bucket_cnt[ow * SPG_CNT_STRIDE], (unsigned long long)cnt); }
         if (tid < 32) {
             unsigned int carry = 0;
             for (int base = 0; base < G; base += 32) {
@@ -1380,23 +1367,11 @@ __global__ void __launch_bounds__(SPG_TTHREADS, SPG_TCTAS) spg_partition_tma_ker
             stage_owner[p] = (unsigned char)o[r];
         }
         // publish run start minus local start, so the copy-out computes its destination with one add
-        if (STATIC) {  // no global atomic: the segment is private to this CTA
-            if (tid >= SPG_TTHREADS - G) { int ow = tid - (SPG_TTHREADS - G); cbase[ow] = cursor[ow] - lbase[ow]; cursor[ow] += hist[ow]; }
-        } else {
-            if (tid >= SPG_TTHREADS - G) { int ow = tid - (SPG_TTHREADS - G); gbase[ow] = my_gbase - lbase[ow]; }
-        }
+        if (tid >= SPG_TTHREADS - G) { int ow = tid - (SPG_TTHREADS - G); gbase[ow] = my_gbase - lbase[ow]; }
         __syncthreads();  // raw buffer b is free from here on
         if (SPG_TBUFS == 1 && tn < n_tiles) issue(tn, 0);  // single buffer: the next tile streams in during the copy-out
         const unsigned int n_tile = lbase[G];
         for (unsigned int p = tid; p < n_tile; p += SPG_TTHREADS) {
-            if (STATIC) {
-                const unsigned int sow = stage_owner[p];
-                const unsigned int soff = cbase[sow] + p;
-                const longlong2 srow = stage[p];
-                if (soff < (unsigned int)a.bucket_cap) a.bucket[((size_t)sow * a.n_cta + blockIdx.x) * a.bucket_cap + soff] = srow;
-                else spg_direct_apply<HAS_SUM, HAS_CNT>(a, srow.x, (unsigned long long)srow.y, 1ull);
-                continue;
-            }
             unsigned int ow = stage_owner[p];
             unsigned long long off = gbase[ow] + p;
             longlong2 row = stage[p];
@@ -1406,9 +1381,6 @@ __global__ void __launch_bounds__(SPG_TTHREADS, SPG_TCTAS) spg_partition_tma_ker
         for (int j = tid; j < G; j += SPG_TTHREADS) hist[j] = 0;
         __syncthreads();
     }
-    if (STATIC)  // rows this CTA left in each owner's segment (rows beyond the segment went the direct way)
-        for (int j = tid; j < G; j += SPG_TTHREADS)
-            a.sub_cnt[(size_t)j * a.n_cta + blockIdx.x] = cursor[j] < (unsigned int)a.bucket_cap ? cursor[j] : (unsigned int)a.bucket_cap;
     if (hot_on) {  // this CTA's heavy-hitter partials -> global table (n_hot atomics per CTA)
         __syncthreads();
         for (int s = tid; s < SPG_HOT_SLOTS; s += SPG_TTHREADS)
@@ -1426,7 +1398,7 @@ __global__ void __launch_bounds__(SPG_TTHREADS, SPG_TCTAS) spg_partition_tma_ker
 // (~2 % at this load: linear-probing stash behind the buckets), a full stash (direct global path), a non-zero high word
 // of the sum — is parked and handled once per iteration behind the hot path.  Two racing inserts may put one key into
 // both of its buckets: harmless, both partial sums are flushed into the same global group.
-template <bool HAS_SUM, bool HAS_CNT, bool STATIC = false, bool INPUT = false>
+template <bool HAS_SUM, bool HAS_CNT>
 __global__ void __launch_bounds__(SPG_THREADS, 1) spg_aggregate_kernel(const __grid_constant__ SpgArgs a) {
     extern __shared__ __align__(16) unsigned char smem_raw[];
     const int NS = a.ns, NT = a.ns + SPG_STASH, tid = threadIdx.x, me = blockIdx.x;  // NS bucket slots + stash
@@ -1437,12 +1409,7 @@ __global__ void __launch_bounds__(SPG_THREADS, 1) spg_aggregate_kernel(const __g
     unsigned int* slo = (unsigned int*)(skeys + NT);  // NT x 4
     unsigned int* scnt = slo + NT;
     const unsigned int NB = (unsigned int)NS / 2;
-#ifdef SPG_K2_NP1  // scratch/spg_harness experiment: single-pass kernel, the per-row pass test is compiled out
-    constexpr unsigned int NP = 1;
-    const unsigned int GP = (unsigned int)gridDim.x;
-#else
     const unsigned int NP = (unsigned int)a.n_pass, GP = (unsigned int)gridDim.x * NP;
-#endif
 
     auto buckets = [&](long long key, unsigned int& b1, unsigned int& b2) {
         const uint64_t h = spg_hash(key);
@@ -1499,54 +1466,19 @@ __global__ void __launch_bounds__(SPG_THREADS, 1) spg_aggregate_kernel(const __g
         add(s, key, val);
     };
 
-    // INPUT (one-pass variant for a few thousand groups, experimental, B200_SPG_ONEPASS=1): no K1 and no owner buckets —
-    // every CTA aggregates a contiguous slice of the INPUT columns in its own table (which then holds all groups).
-    const int64_t in_per = INPUT ? ((((a.n_rows + gridDim.x - 1) / gridDim.x) + 1) & ~1ll) : 0;  // even: 16-byte loads
-    const int64_t in_lo = (int64_t)me * in_per;
-    const int64_t in_n = INPUT ? (a.n_rows - in_lo < 0 ? 0 : (a.n_rows - in_lo < in_per ? a.n_rows - in_lo : in_per)) : 0;
-    const long long* ikeys = INPUT ? a.keys + in_lo : nullptr;
-    const long long* ivals = (INPUT && HAS_SUM) ? a.vals + in_lo : nullptr;
-    unsigned long long n_in = (STATIC || INPUT) ? 0ull : a.bucket_cnt[me * SPG_CNT_STRIDE];
+    unsigned long long n_in = a.bucket_cnt[me * SPG_CNT_STRIDE];
     if (n_in > (unsigned long long)a.bucket_cap) n_in = (unsigned long long)a.bucket_cap;
-    unsigned int* seg_cnt = scnt + NT + 4;  // STATIC: rows in each K1 CTA's segment of this owner's bucket (behind the table)
-    if (STATIC) {
-        for (int i = tid; i < a.n_cta; i += SPG_THREADS) seg_cnt[i] = a.sub_cnt[(size_t)me * a.n_cta + i];
-        __syncthreads();
-    }
     const longlong2* src = a.bucket + (size_t)me * a.bucket_cap;
     constexpr int U = 4;  // independent bucket loads in flight per thread
-    // rows of this thread: rsrc[first + u * stride], u = 0..U-1, valid while < limit
-    auto process = [&](const longlong2* rsrc, unsigned long long first, unsigned long long stride, unsigned long long limit, unsigned int pass, auto full_tag) {
+    // rows of this thread: src[first + u * SPG_THREADS], u = 0..U-1, valid while < n_in
+    auto process = [&](unsigned long long first, unsigned int pass, auto full_tag) {
         constexpr bool FULL = decltype(full_tag)::value;  // FULL: all U rows of every thread are in range (no padding checks)
         longlong2 row[U];
         int sl[U];
-        if (INPUT) {
-            // units of two adjacent rows (first / stride count units, limit counts rows): 16-byte loads from both columns;
-            // a real row whose key equals the free-slot marker goes the direct way here (K1 does that for the bucket path)
 #pragma unroll
-            for (int j = 0; j < U / 2; j++) {
-                const unsigned long long r = 2 * (first + (unsigned long long)j * stride);
-                row[2 * j] = row[2 * j + 1] = make_longlong2(EMPTY_KEY, 0);
-                if (FULL || r + 1 < limit) {
-                    const longlong2 kk = __ldcs(reinterpret_cast<const longlong2*>(ikeys + r));
-                    longlong2 vv = make_longlong2(0, 0);
-                    if (HAS_SUM) vv = __ldcs(reinterpret_cast<const longlong2*>(ivals + r));
-                    row[2 * j] = make_longlong2(kk.x, vv.x);
-                    row[2 * j + 1] = make_longlong2(kk.y, vv.y);
-                    if (kk.x == EMPTY_KEY) spg_direct_apply<HAS_SUM, HAS_CNT>(a, kk.x, (unsigned long long)vv.x, 1ull);
-                    if (kk.y == EMPTY_KEY) spg_direct_apply<HAS_SUM, HAS_CNT>(a, kk.y, (unsigned long long)vv.y, 1ull);
-                } else if (r < limit) {
-                    const long long k0 = ikeys[r], v0 = HAS_SUM ? ivals[r] : 0;
-                    row[2 * j] = make_longlong2(k0, v0);
-                    if (k0 == EMPTY_KEY) spg_direct_apply<HAS_SUM, HAS_CNT>(a, k0, (unsigned long long)v0, 1ull);
-                }
-            }
-        } else {
-#pragma unroll
-            for (int u = 0; u < U; u++) {
-                unsigned long long p = first + (unsigned long long)u * stride;
-                row[u] = (FULL || p < limit) ? __ldcs(rsrc + p) : make_longlong2(EMPTY_KEY, 0);
-            }
+        for (int u = 0; u < U; u++) {
+            unsigned long long p = first + (unsigned long long)u * SPG_THREADS;
+            row[u] = (FULL || p < n_in) ? __ldcs(src + p) : make_longlong2(EMPTY_KEY, 0);
         }
 #pragma unroll
         for (int u = 0; u < U; u++) {  // hot lookups: branch-free
@@ -1556,7 +1488,7 @@ __global__ void __launch_bounds__(SPG_THREADS, 1) spg_aggregate_kernel(const __g
             const ulonglong2 k2 = *reinterpret_cast<const ulonglong2*>(skeys + 2 * b2);
             const unsigned long long uk = (unsigned long long)row[u].x;
             sl[u] = k1.x == uk ? (int)(2 * b1) : k1.y == uk ? (int)(2 * b1 + 1) : k2.x == uk ? (int)(2 * b2) : k2.y == uk ? (int)(2 * b2 + 1) : -1;
-            if ((!FULL || INPUT) && row[u].x == EMPTY_KEY) sl[u] = -2;  // padding lane (INPUT: also marker-key rows, handled above)
+            if (!FULL && row[u].x == EMPTY_KEY) sl[u] = -2;  // padding lane
             // multi-pass: owner = mulhi(hash_hi, G) = mulhi(hash_hi, G * NP) / NP; this pass keeps sub-range `pass` only
             if (NP > 1 && __umulhi((unsigned int)(spg_hash(row[u].x) >> 32), GP) - (unsigned int)me * NP != pass) sl[u] = -2;
         }
@@ -1577,73 +1509,8 @@ __global__ void __launch_bounds__(SPG_THREADS, 1) spg_aggregate_kernel(const __g
     for (unsigned int pass = 0; pass < NP; pass++) {
         for (int s = tid; s < NT; s += SPG_THREADS) { skeys[s] = EMPTY_KEY; slo[s] = 0x80000000u; scnt[s] = 0; }
         __syncthreads();
-        if constexpr (INPUT) {
-            const unsigned long long ustep = (unsigned long long)(U / 2) * SPG_THREADS;          // units per CTA iteration
-            const unsigned long long full_units = (unsigned long long)in_n / (2 * ustep) * ustep;  // iterations with every row in range
-            for (unsigned long long ub = 0; ub < full_units; ub += ustep) process(nullptr, ub + tid, (unsigned long long)SPG_THREADS, (unsigned long long)in_n, pass, std::true_type{});
-            for (unsigned long long ub = full_units; 2 * ub < (unsigned long long)in_n; ub += ustep) process(nullptr, ub + tid, (unsigned long long)SPG_THREADS, (unsigned long long)in_n, pass, std::false_type{});
-        } else if (STATIC) {
-            // every warp streams whole 128-row chunks of the per-(K1 CTA) segments of this owner's bucket: no CTA-wide
-            // iteration, the warps drift apart freely
-            const unsigned int NC = (unsigned int)a.n_cta, C = (unsigned int)a.bucket_cap, CH = (C + 32 * U - 1) / (32 * U);
-            const unsigned int lane = (unsigned int)tid & 31u;
-            for (unsigned int item = (unsigned int)tid >> 5; item < NC * CH; item += SPG_THREADS / 32) {
-                const unsigned int sub = item / CH, r0 = (item - sub * CH) * (32 * U);
-                const unsigned int n = seg_cnt[sub];
-                if (r0 >= n) continue;
-                const longlong2* seg = a.bucket + ((size_t)me * NC + sub) * C + r0;
-                if (r0 + 32 * U <= n) process(seg, lane, 32ull, (unsigned long long)(n - r0), pass, std::true_type{});
-                else process(seg, lane, 32ull, (unsigned long long)(n - r0), pass, std::false_type{});
-            }
-        } else {
-#ifdef SPG_K2_PIPE
-            // scratch/spg_harness experiment: software pipeline — the next UP rows of every thread are in flight while the
-            // current UP rows are aggregated (same register budget as U = 4 rows loaded at once)
-            constexpr int UP = 2;
-            const unsigned long long pstep = (unsigned long long)UP * SPG_THREADS;
-            longlong2 cur[UP], nxt[UP];
-#pragma unroll
-            for (int u = 0; u < UP; u++) {
-                const unsigned long long p = tid + (unsigned long long)u * SPG_THREADS;
-                cur[u] = p < n_in ? __ldcs(src + p) : make_longlong2(EMPTY_KEY, 0);
-            }
-            for (unsigned long long base = 0; base < n_in; base += pstep) {
-#pragma unroll
-                for (int u = 0; u < UP; u++) {
-                    const unsigned long long p = base + pstep + tid + (unsigned long long)u * SPG_THREADS;
-                    nxt[u] = p < n_in ? __ldcs(src + p) : make_longlong2(EMPTY_KEY, 0);
-                }
-                int sl[UP];
-#pragma unroll
-                for (int u = 0; u < UP; u++) {
-                    unsigned int b1, b2;
-                    buckets(cur[u].x, b1, b2);
-                    const ulonglong2 k1 = *reinterpret_cast<const ulonglong2*>(skeys + 2 * b1);
-                    const ulonglong2 k2 = *reinterpret_cast<const ulonglong2*>(skeys + 2 * b2);
-                    const unsigned long long uk = (unsigned long long)cur[u].x;
-                    sl[u] = k1.x == uk ? (int)(2 * b1) : k1.y == uk ? (int)(2 * b1 + 1) : k2.x == uk ? (int)(2 * b2) : k2.y == uk ? (int)(2 * b2 + 1) : -1;
-                    if (cur[u].x == EMPTY_KEY) sl[u] = -2;
-                    if (NP > 1 && __umulhi((unsigned int)(spg_hash(cur[u].x) >> 32), GP) - (unsigned int)me * NP != pass) sl[u] = -2;
-                }
-                long long pk = 0, pv = 0;
-                bool parked = false;
-#pragma unroll
-                for (int u = 0; u < UP; u++) {
-                    if (sl[u] >= 0) add(sl[u], cur[u].x, cur[u].y);
-                    else if (sl[u] == -1) {
-                        if (!parked) { pk = cur[u].x; pv = cur[u].y; parked = true; }
-                        else slow_upsert(cur[u].x, cur[u].y);
-                    }
-                }
-                if (parked) slow_upsert(pk, pv);
-#pragma unroll
-                for (int u = 0; u < UP; u++) cur[u] = nxt[u];
-            }
-#else
-            for (unsigned long long base = 0; base < n_full; base += step) process(src, base + tid, (unsigned long long)SPG_THREADS, n_in, pass, std::true_type{});
-            if (n_full < n_in) process(src, n_full + tid, (unsigned long long)SPG_THREADS, n_in, pass, std::false_type{});
-#endif
-        }
+        for (unsigned long long base = 0; base < n_full; base += step) process(base + tid, pass, std::true_type{});
+        if (n_full < n_in) process(n_full + tid, pass, std::false_type{});
         __syncthreads();
         // flush the shared table into the state's global table
         for (int s = tid; s < NT; s += SPG_THREADS) {
@@ -1658,7 +1525,6 @@ __global__ void __launch_bounds__(SPG_THREADS, 1) spg_aggregate_kernel(const __g
 
 #include "spgn.cuh"  // SPG-N: narrow (int32 key, int32 value) bucket rows: 32 instead of 48 B/row of HBM traffic
 #include "spgg.cuh"  // SPG-G: the same two kernels for nullable / 4-byte / mean / min / max signatures
-#include "spf.cuh"  // SPF: the fused persistent variant of the SM-partitioned path (one kernel, bucket hand-off through L2)
 
 // ---- low-cardinality kernel (LC): every CTA keeps a private shared-memory table of ALL groups ----------------
 // Used when the (estimated) number of groups fits one CTA's table (<= LC_SLOTS / 2), e.g. BASELINE.json configs[0]
@@ -2169,31 +2035,6 @@ class GroupbyState {
                              (const void*)spg_partition_tma_kernel<false, true, true>};
         for (auto f : hf)
             if (cudaFuncSetAttribute(f, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)spg_tma_smem(true)) != cudaSuccess) { cudaGetLastError(); return false; }
-        {   // experimental one-pass variant for a few thousand groups (K2's table over the input columns, no K1)
-            const char* e6 = getenv("B200_SPG_ONEPASS");
-            spg_onepass = e6 && e6[0] == '1';
-            if (spg_onepass) {
-                const void* of[3] = {(const void*)spg_aggregate_kernel<true, true, false, true>, (const void*)spg_aggregate_kernel<true, false, false, true>,
-                                     (const void*)spg_aggregate_kernel<false, true, false, true>};
-                for (auto f : of)
-                    if (cudaFuncSetAttribute(f, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)spg_smem) != cudaSuccess) { cudaGetLastError(); return false; }
-            }
-        }
-        {   // experimental STATIC variant (private (owner, CTA) segments instead of run-reservation atomics)
-            const char* e5 = getenv("B200_SPG_STATIC");
-            spg_static = e5 && e5[0] == '1';
-            if (spg_static) {
-                const void* sf[6] = {(const void*)spg_partition_tma_kernel<true, true, false, true>, (const void*)spg_partition_tma_kernel<true, false, false, true>,
-                                     (const void*)spg_partition_tma_kernel<false, true, false, true>, (const void*)spg_partition_tma_kernel<true, true, true, true>,
-                                     (const void*)spg_partition_tma_kernel<true, false, true, true>, (const void*)spg_partition_tma_kernel<false, true, true, true>};
-                for (auto f : sf)
-                    if (cudaFuncSetAttribute(f, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)spg_tma_smem(true)) != cudaSuccess) { cudaGetLastError(); return false; }
-                const void* af[3] = {(const void*)spg_aggregate_kernel<true, true, true>, (const void*)spg_aggregate_kernel<true, false, true>,
-                                     (const void*)spg_aggregate_kernel<false, true, true>};
-                for (auto f : af)
-                    if (cudaFuncSetAttribute(f, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)spg_smem) != cudaSuccess) { cudaGetLastError(); return false; }
-            }
-        }
         { const char* e2 = getenv("B200_SPG_TMA"); spg_use_tma = !(e2 && e2[0] == '0'); }
         {   // SPG-N (spgn.cuh): narrow bucket rows
             spgn_ns = ((int)(((size_t)max_smem - 256) / 12) - SPG_STASH) & ~1;  // (K2n also has a few static shared words)
@@ -2254,12 +2095,6 @@ class GroupbyState {
     bool spgg_enabled = true;      // B200_SPG_GEN=0 disables the generic SM-partitioned path
     int64_t spgg_launches = 0;
     int spg_n_hot = 0;
-    bool spg_static = false;   // B200_SPG_STATIC=1
-    bool spg_onepass = false;  // B200_SPG_ONEPASS=1
-    // groups one CTA's table takes at ~45 % load: the one-pass variant keeps ALL groups in every CTA
-    int64_t spg_onepass_groups() const { return (int64_t)spg_ns * 45 / 100; }
-    PooledBuf d_sub_cnt;       // STATIC: [owners][K1 CTAs] rows per segment
-    static constexpr int SPG_STATIC_CNT_SLOTS = 128;  // table slots given up for the segment counters (512 x 4 B)
     bool spg_hot_enabled = true, spg_hot_sampled = false;  // heavy-hitter table: sampled once per state, at its first SPG launch
     DevBuf d_hot;                                           // [SPG_HOT_SLOTS] keys + n_hot (int)
     int spg_passes = 1;
@@ -2347,7 +2182,7 @@ class GroupbyState {
             launches++;
         }
         // narrow bucket rows are half the bytes: twice the rows per launch for the same scratch, half the per-launch flushes
-        const bool narrow_call = spgn_enabled && !lowcard && tma_all && !spg_static && spg_n_hot == 0 && spg_sample_wide == 0;
+        const bool narrow_call = spgn_enabled && !lowcard && tma_all && spg_n_hot == 0 && spg_sample_wide == 0;
         const int64_t launch_rows = narrow_call ? 2 * SPG_LAUNCH_ROWS : SPG_LAUNCH_ROWS;
         int64_t li = 0;
         for (int64_t r0 = 0; r0 < n; r0 += launch_rows, li++) {
@@ -2357,19 +2192,9 @@ class GroupbyState {
             // after the table grew (spg_finish), exactly like rows of the direct path
             // uniform keys put rows / owners rows in every bucket (sd = sqrt of that); 12.5 % + 4096 rows head room,
             // anything beyond (skew) takes the direct path inside K1
-            int64_t bucket_cap = (rows / spg_owners) + (rows / spg_owners) / 8 + 4096;
-            const int64_t n_tiles = (rows + SPG_TILE - 1) / SPG_TILE;
-            const int g2s = (int)std::min<int64_t>((int64_t)sms * SPG_TCTAS, n_tiles);  // K1 grid of the TMA variants
-            const bool use_static = spg_static && !lowcard && spg_use_tma && g2s <= 4 * SPG_STATIC_CNT_SLOTS &&
-                                    (((uintptr_t)(keys + r0)) & 15) == 0 && (vals == nullptr || (((uintptr_t)(vals + r0)) & 15) == 0);
-            if (use_static) {
-                // segment of one (owner, K1 CTA) pair: that CTA's share of the rows / owners, + 6 sigma + slack, 128-byte multiple
-                const double mean = (double)((n_tiles + g2s - 1) / g2s) * SPG_TILE / spg_owners;
-                bucket_cap = ((int64_t)(mean + 6.0 * std::sqrt(mean) + 64.0) + 7) & ~7ll;
-            }
+            const int64_t bucket_cap = (rows / spg_owners) + (rows / spg_owners) / 8 + 4096;
             double ta = now();
-            d_bucket.ensure(device, (size_t)spg_owners * (use_static ? (size_t)g2s : 1) * bucket_cap * 16);  // K2 of the previous launch precedes K1 of this one in stream order
-            if (use_static) d_sub_cnt.ensure(device, (size_t)spg_owners * g2s * 4);
+            d_bucket.ensure(device, (size_t)spg_owners * bucket_cap * 16);  // K2 of the previous launch precedes K1 of this one in stream order
             d_retry2[slot].ensure(device, ((size_t)rows + (size_t)spg_owners * spg_ns) * 32);
             t_alloc += now() - ta;
             B200_CUDA(cudaMemsetAsync(d_bucket_cnt.p, 0, (size_t)spg_owners * SPG_CNT_STRIDE * 8, stream));
@@ -2385,13 +2210,7 @@ class GroupbyState {
             a.sum_first = (sum_j >= 0 && cnt_j >= 0 && sum_j < cnt_j) ? 1 : 0; a.ns = spg_ns; a.n_pass = spg_passes;
             cudaEvent_t ev0 = nullptr, ev1 = nullptr;
             if (profiling) { B200_CUDA(cudaEventCreate(&ev0)); B200_CUDA(cudaEventCreate(&ev1)); B200_CUDA(cudaEventRecord(ev0, stream)); }
-            if (!lowcard && spg_onepass && est_groups > 0 && est_groups <= spg_onepass_groups()) {
-                a.n_pass = 1;
-                if (sum_j >= 0 && cnt_j >= 0) spg_aggregate_kernel<true, true, false, true><<<spg_owners, SPG_THREADS, spg_smem, stream>>>(a);
-                else if (sum_j >= 0) spg_aggregate_kernel<true, false, false, true><<<spg_owners, SPG_THREADS, spg_smem, stream>>>(a);
-                else spg_aggregate_kernel<false, true, false, true><<<spg_owners, SPG_THREADS, spg_smem, stream>>>(a);
-                launches--;  // one kernel, the accounting below adds two
-            } else if (lowcard) {
+            if (lowcard) {
                 const bool small = lowcard_small;
                 int gl = (int)std::min<int64_t>((int64_t)sms * (small ? 3 : 2), (rows + LC_THREADS * 2 - 1) / (LC_THREADS * 2));
                 size_t lsm = (size_t)(small ? LC_SLOTS_SMALL : LC_SLOTS_BIG) * 20 + 64;
@@ -2413,7 +2232,7 @@ class GroupbyState {
                 if (hot) { a.hot_tab = d_hot.as<long long>(); a.n_hot = (const int*)(d_hot.as<long long>() + SPG_HOT_SLOTS); }
                 const size_t tsm = spg_tma_smem(hot);
                 // SPG-N: the sample found only rows that fit (int32 key, int32 value), and the rows that did not so far are rare
-                const bool narrow = spgn_enabled && tma && !hot && !use_static && spg_sample_wide == 0 && spgn_wide_rows * 64 <= rows_consumed;
+                const bool narrow = spgn_enabled && tma && !hot && spg_sample_wide == 0 && spgn_wide_rows * 64 <= rows_consumed;
                 if (narrow) {
                     a.ns = spgn_ns;
                     // first flush into an empty table: per-CTA ticket reservation, but only with >= 25 % head room under the group
@@ -2430,20 +2249,6 @@ class GroupbyState {
                     else if (sum_j >= 0) { spgn_partition_kernel<true, false><<<g2, SPG_TTHREADS, nsm, stream>>>(a); spgn_aggregate_kernel<true, false><<<spg_owners, SPG_THREADS, spgn_smem, stream>>>(a); }
                     else { spgn_partition_kernel<false, true><<<g2, SPG_TTHREADS, nsm, stream>>>(a); spgn_aggregate_kernel<false, true><<<spg_owners, SPG_THREADS, spgn_smem, stream>>>(a); }
                     spgn_launches++;
-                } else
-                if (use_static) {
-                    a.sub_cnt = d_sub_cnt.as<unsigned int>(); a.n_cta = g2; a.ns = spg_ns - SPG_STATIC_CNT_SLOTS;
-                    const size_t ssm = spg_tma_smem(true);
-#define B200_SPG_STATIC_LAUNCH(S, C)                                                                                      \
-    do {                                                                                                                  \
-        if (hot) spg_partition_tma_kernel<S, C, true, true><<<g2, SPG_TTHREADS, ssm, stream>>>(a);                        \
-        else spg_partition_tma_kernel<S, C, false, true><<<g2, SPG_TTHREADS, ssm, stream>>>(a);                           \
-        spg_aggregate_kernel<S, C, true><<<spg_owners, SPG_THREADS, spg_smem, stream>>>(a);                               \
-    } while (0)
-                    if (sum_j >= 0 && cnt_j >= 0) B200_SPG_STATIC_LAUNCH(true, true);
-                    else if (sum_j >= 0) B200_SPG_STATIC_LAUNCH(true, false);
-                    else B200_SPG_STATIC_LAUNCH(false, true);
-#undef B200_SPG_STATIC_LAUNCH
                 } else if (sum_j >= 0 && cnt_j >= 0) {
                     if (hot) spg_partition_tma_kernel<true, true, true><<<g2, SPG_TTHREADS, tsm, stream>>>(a);
                     else if (tma) spg_partition_tma_kernel<true, true><<<g2, SPG_TTHREADS, tsm, stream>>>(a);

@@ -12,11 +12,8 @@
 #pragma once
 
 constexpr int SPGN_EMPTY = (int)0x80000000;
-#ifndef SPGN_TILE_ROWS
-#define SPGN_TILE_ROWS 4096
-#endif
-constexpr int SPGN_TILE = SPGN_TILE_ROWS;            // rows per K1n tile (8-byte staged rows leave room for twice the 16-byte kernels' tile)
-constexpr int SPGN_CTAS = SPGN_TILE == 4096 ? 2 : 3;  // K1n CTAs per SM
+constexpr int SPGN_TILE = 4096;  // rows per K1n tile (8-byte staged rows leave room for twice the 16-byte kernels' tile)
+constexpr int SPGN_CTAS = 2;     // K1n CTAs per SM
 
 // find-or-insert for a caller that already holds a group ticket: `inserted` says whether THIS call created the group (else the
 // ticket goes back).  The table cannot be full: tickets bound the number of groups by cap / 2.

@@ -1,11 +1,10 @@
 // spg_harness.cu — times the SPG kernel pair (K1 spg_partition_tma_kernel, K2 spg_aggregate_kernel) in isolation, outside
-// the operator state machine, so kernel variants can be compared with one short GPU run each.  Development tool, not part
+// the operator state machine, so a kernel change can be timed with one short GPU run.  Development tool, not part
 // of the library: it includes groupby.cu to reach the kernels and links misc.cu for the buffer pool.
 //
 //   nvcc -gencode arch=compute_100a,code=sm_100a -O3 -lineinfo -std=c++17 -I bodo_b200/csrc \
 //        scratch/spg_harness.cu bodo_b200/csrc/misc.cu -o scratch/spg_harness
-//   scratch/spg_harness [log2_rows=27] [groups=1000000] [reps=5] [mode=0] [cnt_stride_pad_bytes=0]
-//       mode 0 = shipping K1 + K2, 1 = STATIC variant, 2 = one-pass variant (K2 over the input columns, no K1; use <= 6000 groups)
+//   scratch/spg_harness [log2_rows=27] [groups=1000000] [reps=5] [cnt_stride_pad_bytes=0]
 //
 // Prints per-kernel CUDA-event times (min / median over reps), the achieved fraction of the 16 B/row stream roofline for the
 // pair, and checks SUM/COUNT totals against the input (result must be exact).
@@ -40,9 +39,7 @@ int main(int argc, char** argv) {
     const int lg = argc > 1 ? atoi(argv[1]) : 27;
     const uint64_t groups = argc > 2 ? strtoull(argv[2], nullptr, 10) : 1000000ull;
     const int reps = argc > 3 ? atoi(argv[3]) : 5;
-    const int mode = argc > 4 ? atoi(argv[4]) : 0;
-    const bool use_static = mode == 1, onepass = mode == 2;
-    const size_t pad = argc > 5 ? strtoull(argv[5], nullptr, 10) : 0;  // shifts the owner row counters inside their allocation
+    const size_t pad = argc > 4 ? strtoull(argv[4], nullptr, 10) : 0;  // shifts the owner row counters inside their allocation
     const int64_t rows = 1ll << lg;
     int dev = 0, sms = 0, max_smem = 0;
     CK(cudaSetDevice(dev));
@@ -51,26 +48,20 @@ int main(int argc, char** argv) {
     const int owners = sms;
     int ns = ((int)(((size_t)max_smem - 64) / 16) - SPG_STASH) & ~1;
     const size_t k2_smem = (size_t)(ns + SPG_STASH) * 16 + 16;
-    const size_t k1_smem = GroupbyState::spg_tma_smem(use_static);
+    const size_t k1_smem = GroupbyState::spg_tma_smem();
     const int64_t n_tiles = (rows + SPG_TILE - 1) / SPG_TILE;
     const int g1 = (int)std::min<int64_t>((int64_t)sms * SPG_TCTAS, n_tiles);
 
     long long *keys, *vals, *tkeys, *counters;
     unsigned long long *acc_sum, *acc_cnt, *bucket_cnt_raw, *retry, *chk;
     longlong2* bucket;
-    unsigned int* sub_cnt;
     const uint64_t cap = 1ull << 22;
     CK(cudaMalloc(&keys, rows * 8)); CK(cudaMalloc(&vals, rows * 8));
     CK(cudaMalloc(&tkeys, (cap + 2) * 8)); CK(cudaMalloc(&acc_sum, (cap + 2) * 8)); CK(cudaMalloc(&acc_cnt, (cap + 2) * 8));
     CK(cudaMalloc(&counters, 64)); CK(cudaMalloc(&chk, 16));
-    int64_t bucket_cap = rows / owners + rows / owners / 8 + 4096;
-    if (use_static) {
-        const double mean = (double)((n_tiles + g1 - 1) / g1) * SPG_TILE / owners;
-        bucket_cap = ((int64_t)(mean + 6.0 * sqrt(mean) + 64.0) + 7) & ~7ll;
-    }
-    CK(cudaMalloc(&bucket, (size_t)owners * (use_static ? g1 : 1) * bucket_cap * 16));
+    const int64_t bucket_cap = rows / owners + rows / owners / 8 + 4096;
+    CK(cudaMalloc(&bucket, (size_t)owners * bucket_cap * 16));
     CK(cudaMalloc(&bucket_cnt_raw, (size_t)owners * SPG_CNT_STRIDE * 8 + pad + 256));
-    CK(cudaMalloc(&sub_cnt, (size_t)owners * g1 * 4 + 16));
     CK(cudaMalloc(&retry, ((size_t)rows + (size_t)owners * ns) * 32));
     unsigned long long* bucket_cnt = (unsigned long long*)((char*)bucket_cnt_raw + pad);
     harness_fill_kernel<<<sms * 8, 256>>>(keys, vals, rows, groups);
@@ -82,14 +73,10 @@ int main(int argc, char** argv) {
     a.keys = keys; a.vals = vals; a.n_rows = rows; a.n_owners = owners;
     a.tkeys = tkeys; a.cap = cap; a.acc_sum = acc_sum; a.acc_cnt = acc_cnt; a.counters = counters; a.group_limit = (long long)(cap / 2);
     a.bucket = bucket; a.bucket_cnt = bucket_cnt; a.bucket_cap = bucket_cap; a.retry = retry; a.retry_ctr = counters + 1;
-    a.sum_first = 1; a.ns = use_static ? ns - GroupbyState::SPG_STATIC_CNT_SLOTS : ns; a.n_pass = 1;
-    a.sub_cnt = sub_cnt; a.n_cta = g1;
+    a.sum_first = 1; a.ns = ns; a.n_pass = 1;
 
-    auto k1 = use_static ? (const void*)spg_partition_tma_kernel<true, true, false, true> : (const void*)spg_partition_tma_kernel<true, true, false, false>;
-    auto k2 = use_static ? (const void*)spg_aggregate_kernel<true, true, true> : (const void*)spg_aggregate_kernel<true, true, false>;
-    CK(cudaFuncSetAttribute(k1, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)k1_smem));
-    CK(cudaFuncSetAttribute(k2, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)k2_smem));
-    CK(cudaFuncSetAttribute((const void*)spg_aggregate_kernel<true, true, false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)k2_smem));
+    CK(cudaFuncSetAttribute((const void*)spg_partition_tma_kernel<true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)k1_smem));
+    CK(cudaFuncSetAttribute((const void*)spg_aggregate_kernel<true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)k2_smem));
 
     std::vector<float> t1, t2;
     cudaEvent_t e0, e1, e2;
@@ -97,13 +84,9 @@ int main(int argc, char** argv) {
     for (int r = 0; r < reps + 1; r++) {  // the first repetition (table inserts, cold) is not reported
         CK(cudaMemsetAsync(bucket_cnt, 0, (size_t)owners * SPG_CNT_STRIDE * 8));
         CK(cudaEventRecord(e0));
-        if (onepass) {}
-        else if (use_static) spg_partition_tma_kernel<true, true, false, true><<<g1, SPG_TTHREADS, k1_smem>>>(a);
-        else spg_partition_tma_kernel<true, true, false, false><<<g1, SPG_TTHREADS, k1_smem>>>(a);
+        spg_partition_tma_kernel<true, true><<<g1, SPG_TTHREADS, k1_smem>>>(a);
         CK(cudaEventRecord(e1));
-        if (onepass) spg_aggregate_kernel<true, true, false, true><<<owners, SPG_THREADS, k2_smem>>>(a);
-        else if (use_static) spg_aggregate_kernel<true, true, true><<<owners, SPG_THREADS, k2_smem>>>(a);
-        else spg_aggregate_kernel<true, true, false><<<owners, SPG_THREADS, k2_smem>>>(a);
+        spg_aggregate_kernel<true, true><<<owners, SPG_THREADS, k2_smem>>>(a);
         CK(cudaEventRecord(e2));
         CK(cudaEventSynchronize(e2));
         CK(cudaGetLastError());
@@ -125,12 +108,9 @@ int main(int argc, char** argv) {
     CK(cudaMemcpy(hc, counters, 64, cudaMemcpyDeviceToHost));
     const bool ok = h[0] == (unsigned long long)rows * (reps + 1) && h[1] == hin * (unsigned long long)(reps + 1) && hc[1] == 0;
     const float m1 = t1[t1.size() / 2], m2 = t2[t2.size() / 2];
-    printf("{\"rows\": %lld, \"groups\": %llu, \"mode\": %d, \"k1_ms\": {\"min\": %.4f, \"median\": %.4f}, \"k2_ms\": {\"min\": %.4f, \"median\": %.4f}, "
+    printf("{\"rows\": %lld, \"groups\": %llu, \"k1_ms\": {\"min\": %.4f, \"median\": %.4f}, \"k2_ms\": {\"min\": %.4f, \"median\": %.4f}, "
            "\"pair_grows_per_s\": %.2f, \"roofline_frac\": %.4f, \"table_groups\": %lld, \"retry_rows\": %lld, \"check\": \"%s\"}\n",
-           (long long)rows, (unsigned long long)groups, mode, t1[0], m1, t2[0], m2, rows / ((m1 + m2) * 1e-3) / 1e9,
+           (long long)rows, (unsigned long long)groups, t1[0], m1, t2[0], m2, rows / ((m1 + m2) * 1e-3) / 1e9,
            rows * 16.0 / ((m1 + m2) * 1e-3) / 6574.8e9, hc[0], hc[1], ok ? "ok" : "MISMATCH");
     return ok ? 0 : 3;
 }
-// Variants (compile-time, harness builds only; the library never defines these):
-//   -DSPG_K2_NP1   single-pass K2, per-row pass test compiled out
-//   -DSPG_K2_PIPE  K2 with a 2 + 2 software pipeline of the bucket loads
