@@ -175,6 +175,22 @@ __device__ __forceinline__ uint32_t hash_keys_row(const KeySet& k, int64_t i, ui
     return h;
 }
 
+// Key-tuple tables (multi-key groupby, multi-key join): a slot is claimed through a 64-bit tag word, the hash of the widened
+// int64 key values and the NA mask (bit j = key column j is valid) with bit 63 set, so a published tag is never TAG_EMPTY or
+// TAG_LOCKED.  The claiming thread CASes empty -> locked, writes what readers compare against, fences and publishes the tag.
+constexpr unsigned long long TAG_EMPTY = 0ull, TAG_LOCKED = 1ull;
+
+__device__ __forceinline__ unsigned long long ld_acquire_u64(const unsigned long long* p) {
+    unsigned long long v;
+    asm volatile("ld.acquire.gpu.global.u64 %0, [%1];" : "=l"(v) : "l"(p) : "memory");
+    return v;
+}
+__device__ __forceinline__ unsigned long long mk_tag(const long long* keys, unsigned int mask, int nk) {
+    unsigned long long h = 0x9E3779B97F4A7C15ULL ^ mask;
+    for (int j = 0; j < nk; j++) h = xxh3_64_short((unsigned long long)keys[j] ^ (h * 0xD1B54A32D192ED03ULL), 8, SEED_HASH_PARTITION + j);
+    return h | 0x8000000000000000ULL;
+}
+
 // order-preserving double <-> uint64 encoding (so float min/max are native 64-bit integer atomics)
 __host__ __device__ __forceinline__ uint64_t f64_to_ordered(double d) {
 #ifdef __CUDA_ARCH__

@@ -703,7 +703,6 @@ __global__ void xchg_combine_slab_kernel(const __grid_constant__ CombineArgs a, 
 // Readers that find their own tag compare the full tuple (so the result is exact, the tag only prunes); readers that
 // find `locked` re-read the slot.  Aggregate updates are the single-key kernel's apply_ops.
 constexpr int MAX_KEYS = 4;
-constexpr unsigned long long TAG_EMPTY = 0ull, TAG_LOCKED = 1ull;
 
 struct MkArgs {
     int nk;
@@ -725,16 +724,6 @@ struct MkArgs {
     unsigned long long seq_base;  // unused (first / last are single-key only); apply_ops reads it
 };
 
-__device__ __forceinline__ unsigned long long ld_acquire_u64(const unsigned long long* p) {
-    unsigned long long v;
-    asm volatile("ld.acquire.gpu.global.u64 %0, [%1];" : "=l"(v) : "l"(p) : "memory");
-    return v;
-}
-__device__ __forceinline__ unsigned long long mk_tag(const long long* keys, unsigned int mask, int nk) {
-    unsigned long long h = 0x9E3779B97F4A7C15ULL ^ mask;
-    for (int j = 0; j < nk; j++) h = xxh3_64_short((unsigned long long)keys[j] ^ (h * 0xD1B54A32D192ED03ULL), 8, SEED_HASH_PARTITION + j);
-    return h | 0x8000000000000000ULL;
-}
 template <typename A>
 __device__ __forceinline__ uint64_t find_or_insert_mk(const A& a, const long long* keys, unsigned int mask, unsigned long long tag) {
     const uint64_t m = a.cap - 1;

@@ -17,7 +17,12 @@
 // bodo/pandas/physical/join.h:267): NA joins NA.  false (the default of join_state_init_py_entry, SQL semantics): rows
 // with an NA key never match — they are filtered from the build table unless it is the outer side
 // (_join.cpp:3180 filter_na_values) and only survive as NULL-extended rows of an outer join.
+// Key columns: 1..4 (HashJoinState's n_keys), the first n_keys columns of each side.  One key column uses the key-valued table
+// below; a tuple of 2..4 uses a tag table whose slots point at a representative build row (see "multi-column keys").  With
+// is_na_equal = false a row with an NA in ANY key column matches nothing (filter_na_values works over all keys); with true, NA
+// equals NA at the same key position and never equals a value.
 #include <algorithm>
+#include <type_traits>
 #include <vector>
 
 #include "common.cuh"
@@ -185,6 +190,102 @@ __global__ void join_probe_count_kernel(const void* key_data, int key_ctype, con
             long long key = load_int_as_i64(key_data, key_ctype, i);
             s = key == J_EMPTY ? (uint32_t)cap + 1 : j_find(tkeys, cap, key);
         }
+        uint32_t c = s == J_NONE ? 0 : info[s].cnt;
+        if (c == 0) s = J_NONE;
+        if (mode == 1) { pslot[i] = J_NONE; pcnt[i] = c ? 0u : 1u; continue; }
+        if (mode == 2) { pslot[i] = J_NONE; pcnt[i] = 1u; mark[i] = c ? 1 : 0; continue; }
+        pslot[i] = s;
+        pcnt[i] = c ? c : (probe_outer ? 1u : 0u);
+    }
+}
+
+// ---- multi-column keys (2..4 key columns) ----
+// A tuple maps to a slot through the slot's tag word (mk_tag, common.cuh: 0 = free, 1 = being claimed, bit 63 = published tag of
+// the widened key values + NA mask).  The claiming row writes itself into SlotInfo.first before it publishes the tag, and first is
+// never overwritten: it is the slot's representative row.  A reader that finds its own tag compares the NA mask and every key
+// value with that row in the build columns, which stay on the device for the state's lifetime, so the table holds no key columns.
+// NA is part of the tuple, so there is no NA slot and no free-slot-marker slot.  Everything that only sees slots and row ids
+// (counts, CSR groups, gather, outer tail) is the single-key code.
+constexpr int J_MAX_KEYS = MAX_HASH_KEYS;
+struct JKeys {  // the key columns of one side: validity is one byte per row on the build side, a bitmap on the probe side
+    const void* data[J_MAX_KEYS];
+    const uint8_t* valid[J_MAX_KEYS];
+    int ctype[J_MAX_KEYS];
+};
+// row i's tuple widened to int64 (NA positions read as 0); returns the NA mask, bit j set = key j valid
+template <int NK, bool BYTE_VALID>
+__device__ __forceinline__ unsigned int j_load_tuple(const JKeys& k, int64_t i, long long (&keys)[NK]) {
+    unsigned int mask = 0;
+#pragma unroll
+    for (int j = 0; j < NK; j++) {
+        const bool v = BYTE_VALID ? (k.valid[j] == nullptr || k.valid[j][i] != 0) : bit_valid(k.valid[j], i);
+        keys[j] = v ? (long long)load_int_as_i64(k.data[j], k.ctype[j], i) : 0;
+        mask |= v ? (1u << j) : 0u;
+    }
+    return mask;
+}
+template <int NK>
+__device__ __forceinline__ bool j_tuple_eq(const JKeys& b, uint32_t brow, const long long (&keys)[NK], unsigned int mask) {
+    long long bk[NK];
+    bool eq = j_load_tuple<NK, true>(b, brow, bk) == mask;
+#pragma unroll
+    for (int j = 0; j < NK; j++) eq = eq && bk[j] == keys[j];
+    return eq;
+}
+// BuildHashTable for tuples: the claim protocol of the multi-key groupby (find_or_insert_mk); row_slot as in the single-key kernel
+template <int NK>
+__global__ void join_insert_count_mk_kernel(const __grid_constant__ JKeys b, int64_t n, unsigned long long* tags, uint64_t cap, SlotInfo* info,
+                                            uint32_t* row_slot, int na_equal) {
+    const uint64_t m = cap - 1;
+    int64_t stride = (int64_t)gridDim.x * blockDim.x;
+    for (int64_t i = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; i < n; i += stride) {
+        long long keys[NK];
+        const unsigned int mask = j_load_tuple<NK, true>(b, i, keys);
+        if (!na_equal && mask != (1u << NK) - 1u) { row_slot[i] = J_NONE; continue; }  // an NA in any key column: never matches
+        const unsigned long long tag = mk_tag(keys, mask, NK);
+        uint64_t s = (tag >> 20) & m;
+        while (true) {
+            const unsigned long long t = ld_acquire_u64(tags + s);
+            if (t == tag) {
+                if (j_tuple_eq<NK>(b, __ldcg(&info[s].first), keys, mask)) break;
+            } else if (t == TAG_EMPTY) {
+                if (atomicCAS(tags + s, TAG_EMPTY, TAG_LOCKED) == TAG_EMPTY) {
+                    info[s].first = (uint32_t)i;
+                    __threadfence();
+                    atomicExch(tags + s, tag);  // publish
+                    break;
+                }
+                continue;  // another row claimed the slot meanwhile: look at it again
+            } else if (t == TAG_LOCKED) {
+                continue;  // being claimed: re-read
+            }
+            s = (s + 1) & m;
+        }
+        row_slot[i] = (uint32_t)s;
+        atomicAdd(&info[s].cnt, 1u);
+    }
+}
+template <int NK>
+__device__ __forceinline__ uint32_t j_find_mk(const unsigned long long* __restrict__ tags, uint64_t cap, const SlotInfo* __restrict__ info,
+                                              const JKeys& b, const long long (&keys)[NK], unsigned int mask) {
+    const uint64_t m = cap - 1;
+    const unsigned long long tag = mk_tag(keys, mask, NK);
+    for (uint64_t s = (tag >> 20) & m;; s = (s + 1) & m) {
+        const unsigned long long t = __ldg(tags + s);
+        if (t == tag && j_tuple_eq<NK>(b, info[s].first, keys, mask)) return (uint32_t)s;
+        if (t == TAG_EMPTY) return J_NONE;
+    }
+}
+// probe pass A for tuples: same outputs and modes as join_probe_count_kernel
+template <int NK>
+__global__ void join_probe_count_mk_kernel(const __grid_constant__ JKeys p, const __grid_constant__ JKeys b, int64_t n, const unsigned long long* tags,
+                                           uint64_t cap, const SlotInfo* info, int probe_outer, uint32_t* pslot, uint32_t* pcnt, int na_equal, int mode,
+                                           uint8_t* mark) {
+    int64_t stride = (int64_t)gridDim.x * blockDim.x;
+    for (int64_t i = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; i < n; i += stride) {
+        long long keys[NK];
+        const unsigned int mask = j_load_tuple<NK, false>(p, i, keys);
+        uint32_t s = na_equal || mask == (1u << NK) - 1u ? j_find_mk<NK>(tags, cap, info, b, keys, mask) : J_NONE;
         uint32_t c = s == J_NONE ? 0 : info[s].cnt;
         if (c == 0) s = J_NONE;
         if (mode == 1) { pslot[i] = J_NONE; pcnt[i] = c ? 0u : 1u; continue; }
@@ -426,6 +527,100 @@ __global__ void __launch_bounds__(256) join_probe_fast_kernel(const __grid_const
         __syncthreads();
     }
 }
+// Fused probe for unique build tuples: join_probe_fast_kernel's tiles, cursor and ballot ranks over a Slot16 table whose key word is
+// the tuple's tag.  The packed build row holds every build column, keys first, so the tuple check and the gather read one row.
+struct FastProbeMkArgs {
+    int64_t n_probe;
+    JKeys pk;                                    // probe key columns (bitmaps)
+    const uint8_t* bk_valid[J_MAX_KEYS];         // build key validity (one byte per row), nullptr = all valid
+    unsigned long long bk_bits[J_MAX_KEYS];      // low-bit mask of each key's width: packed fields are zero-extended raw bits
+    const Slot16* slots; uint64_t cap;
+    const unsigned long long* bpack; int n_fields;
+    unsigned long long* cursor;
+    int n_b, n_p;
+    int na_equal;
+    int b_field[J_MAX_COLS];                     // kept build col -> packed field
+    const uint8_t* b_valid[J_MAX_COLS]; int b_size[J_MAX_COLS];
+    const void* p_data[J_MAX_COLS]; const uint8_t* p_valid[J_MAX_COLS]; int p_size[J_MAX_COLS];
+    void* ob_data[J_MAX_COLS]; uint8_t* ob_valid[J_MAX_COLS];
+    void* op_data[J_MAX_COLS]; uint8_t* op_valid[J_MAX_COLS];
+};
+// (the minimum-blocks hint only steers ptxas' allocation: without it the NK = 3 instance spills 16 bytes at 40 registers)
+template <int NK>
+__global__ void __launch_bounds__(256, 4) join_probe_fast_mk_kernel(const __grid_constant__ FastProbeMkArgs a) {
+    constexpr int R = 4, NW = 8, TILE = 256 * R;
+    __shared__ unsigned int wcnt[R * NW];
+    __shared__ unsigned int woff[R * NW];
+    __shared__ unsigned long long tile_base;
+    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+    const uint64_t mask = a.cap - 1;
+    const int64_t n_tiles = (a.n_probe + TILE - 1) / TILE;
+    for (int64_t t = blockIdx.x; t < n_tiles; t += gridDim.x) {
+        uint32_t brow[R];
+        unsigned int rank[R];
+        bool match[R];
+#pragma unroll
+        for (int r = 0; r < R; r++) {
+            const int64_t i = t * TILE + r * 256 + threadIdx.x;
+            match[r] = false; brow[r] = 0;
+            long long keys[NK];
+            const unsigned int na = i < a.n_probe ? j_load_tuple<NK, false>(a.pk, i, keys) : 0u;
+            if (i < a.n_probe && (a.na_equal || na == (1u << NK) - 1u)) {
+                const unsigned long long tag = mk_tag(keys, na, NK);
+                uint64_t s = (tag >> 20) & mask;
+                while (true) {
+                    int4 raw = __ldg(reinterpret_cast<const int4*>(a.slots + s));
+                    const unsigned long long k = (unsigned long long)(unsigned int)raw.x | ((unsigned long long)(unsigned int)raw.y << 32);
+                    if (k == TAG_EMPTY) break;
+                    if (k == tag) {
+                        const uint32_t row = (unsigned int)raw.z;
+                        const unsigned long long* fields = a.bpack + (size_t)row * a.n_fields;
+                        bool eq = true;
+#pragma unroll
+                        for (int j = 0; j < NK; j++) {
+                            const bool bv = a.bk_valid[j] == nullptr || a.bk_valid[j][row] != 0;
+                            eq = eq && bv == (((na >> j) & 1u) != 0) && (!bv || __ldg(fields + j) == ((unsigned long long)keys[j] & a.bk_bits[j]));
+                        }
+                        if (eq) { match[r] = (unsigned int)raw.w > 0; brow[r] = row; break; }
+                    }
+                    s = (s + 1) & mask;
+                }
+            }
+        }
+#pragma unroll
+        for (int r = 0; r < R; r++) {
+            unsigned m = __ballot_sync(0xffffffffu, match[r]);
+            rank[r] = __popc(m & ((1u << lane) - 1));
+            if (lane == 0) wcnt[r * NW + warp] = __popc(m);
+        }
+        __syncthreads();
+        if (warp == 0) {
+            unsigned int x = wcnt[lane], inc = x;
+#pragma unroll
+            for (int d = 1; d < 32; d <<= 1) { unsigned int y = __shfl_up_sync(0xffffffffu, inc, d); if (lane >= d) inc += y; }
+            woff[lane] = inc - x;
+            if (lane == 31) tile_base = inc ? atomicAdd(a.cursor, (unsigned long long)inc) : 0ull;
+        }
+        __syncthreads();
+        const unsigned long long base = tile_base;
+#pragma unroll
+        for (int r = 0; r < R; r++) {
+            if (!match[r]) continue;
+            const int64_t i = t * TILE + r * 256 + threadIdx.x;
+            const int64_t orow = (int64_t)(base + woff[r * NW + warp] + rank[r]);
+            const unsigned long long* fields = a.bpack + (size_t)brow[r] * a.n_fields;
+            for (int k2 = 0; k2 < a.n_b; k2++) {
+                store_sized(a.ob_data[k2], orow, __ldg(fields + a.b_field[k2]), a.b_size[k2]);
+                if (a.ob_valid[k2]) a.ob_valid[k2][orow] = a.b_valid[k2] ? a.b_valid[k2][brow[r]] : 1;
+            }
+            for (int k2 = 0; k2 < a.n_p; k2++) {
+                copy_item(a.op_data[k2], orow, a.p_data[k2], i, a.p_size[k2]);
+                if (a.op_valid[k2]) a.op_valid[k2][orow] = bit_valid(a.p_valid[k2], i) ? 1 : 0;
+            }
+        }
+        __syncthreads();
+    }
+}
 
 // ---- inline-payload probe: the specialisation for all-8-byte, bitmap-free schemas with at most two build payload columns ----
 // Slot32 = {key, f0, f1, first | cnt << 32}: key AND payload of a unique-key build row sit in ONE 32-byte sector, so a probe
@@ -656,6 +851,7 @@ class JoinState {
     int device; cudaStream_t stream; int sms;
     std::vector<int8_t> b_ct, b_at, p_ct, p_at;
     int n_b, n_p;
+    int nk = 1;  // key columns: the first nk columns of each side
     bool build_outer, probe_outer;
     bool na_equal = false;  // is_na_equal of the reference's HashJoinState
     int64_t output_batch_size;
@@ -665,7 +861,7 @@ class JoinState {
     int64_t n_build = 0;
     bool build_final = false;
     uint64_t cap = 0;
-    DevBuf d_tkeys, d_info, d_row_slot, d_cnt_multi, d_goffs, d_groups, d_fill, d_bmatched;
+    DevBuf d_tkeys, d_info, d_row_slot, d_cnt_multi, d_goffs, d_groups, d_fill, d_bmatched;  // d_tkeys: keys, or tuple tags (nk > 1)
     DevBuf d_slots16, d_bpack, d_cursor;  // fast path (unique build keys, inner join)
     DevBuf d_slots32;                      // inline-payload table (all-8-byte bitmap-free build schema, <= 2 payload columns)
     bool fast_ready = false, inline_ready = false;
@@ -692,11 +888,13 @@ class JoinState {
     JoinState(const int8_t* bct, const int8_t* bat, int nb, const int8_t* pct, const int8_t* pat, int np, uint64_t n_keys,
               bool bo, bool po, bool na_eq, int64_t obs, int dev, int64_t expected_build_rows, cudaStream_t st)
         : device(dev), stream(st), n_b(nb), n_p(0), build_outer(bo), probe_outer(po), na_equal(na_eq), output_batch_size(obs) {
-        B200_REQUIRE(n_keys == 1, "b200 join: exactly one key column is supported (multi-key is a 'next' row, SURVEY.md §8f)");
+        B200_REQUIRE(n_keys >= 1 && n_keys <= (uint64_t)J_MAX_KEYS, "b200 join: between 1 and 4 key columns are supported");
+        nk = (int)n_keys;
         B200_REQUIRE(nb >= 1 && np >= 0 && nb <= J_MAX_COLS && np <= J_MAX_COLS, "b200 join: between 1 and 32 columns per side");
+        B200_REQUIRE(nb >= nk, "b200 join: the build table has fewer columns than key columns");
         b_ct.assign(bct, bct + nb); b_at.assign(bat, bat + nb);
         for (int c = 0; c < nb; c++) B200_REQUIRE(ctype_size(b_ct[c]) > 0, "b200 join: unsupported build column dtype");
-        B200_REQUIRE(!ctype_is_float(b_ct[0]), "b200 join: key columns must be integer/date typed");
+        for (int j = 0; j < nk; j++) B200_REQUIRE(!ctype_is_float(b_ct[j]), "b200 join: key columns must be integer/date typed");
         B200_CUDA(cudaSetDevice(device)); scratch_set_stream(stream);
         sms = num_sms(device);
         bcol.resize(nb); bvalid.resize(nb); b_has_valid.assign(nb, false);
@@ -711,14 +909,39 @@ class JoinState {
         B200_REQUIRE(np >= 1 && np <= J_MAX_COLS, "b200 join: between 1 and 32 columns per side");
         p_ct.assign(pct, pct + np); p_at.assign(pat, pat + np); n_p = np;
         for (int c = 0; c < np; c++) B200_REQUIRE(ctype_size(p_ct[c]) > 0, "b200 join: unsupported probe column dtype");
-        B200_REQUIRE(!ctype_is_float(p_ct[0]), "b200 join: key columns must be integer/date typed");
-        B200_REQUIRE(ctype_size(b_ct[0]) == ctype_size(p_ct[0]), "b200 join: build and probe key widths differ");
+        B200_REQUIRE(np >= nk, "b200 join: the probe table has fewer columns than key columns");
+        for (int j = 0; j < nk; j++) {
+            // sharded placement hashes each key's sizeof(T) raw bytes, so both sides must agree on the width at every position
+            B200_REQUIRE(!ctype_is_float(p_ct[j]), "b200 join: key columns must be integer/date typed");
+            B200_REQUIRE(ctype_size(b_ct[j]) == ctype_size(p_ct[j]),
+                         nk == 1 ? std::string("b200 join: build and probe key widths differ")
+                                 : "b200 join: build and probe key widths differ at key position " + std::to_string(j));
+        }
         out_data.resize(n_b + np); out_vbytes.resize(n_b + np); out_bitmap.resize(n_b + np);
         if ((int)stage_data.size() < std::max(n_b, np)) { stage_data.resize(std::max(n_b, np)); stage_valid.resize(std::max(n_b, np)); }
     }
     ~JoinState() { cudaSetDevice(device); scratch_set_stream(stream); cudaStreamSynchronize(stream); pinned_release(h_cursor, 8); }
 
     int grid_for(int64_t n) const { return (int)std::max<int64_t>(1, std::min<int64_t>((n + 255) / 256, (int64_t)sms * 8)); }
+
+    // multi-key kernels are instantiated per key count; f(std::integral_constant<int, NK>) launches one
+    template <typename F> void with_nk(F&& f) const {
+        switch (nk) {
+            case 2: f(std::integral_constant<int, 2>()); break;
+            case 3: f(std::integral_constant<int, 3>()); break;
+            default: f(std::integral_constant<int, 4>()); break;
+        }
+    }
+    JKeys build_keys() const {
+        JKeys k{};
+        for (int j = 0; j < nk; j++) { k.data[j] = bcol[j].buf.p; k.valid[j] = b_has_valid[j] ? bvalid[j].buf.as<uint8_t>() : nullptr; k.ctype[j] = b_ct[j]; }
+        return k;
+    }
+    JKeys probe_keys(const std::vector<const void*>& data, const std::vector<const uint8_t*>& valid) const {
+        JKeys k{};
+        for (int j = 0; j < nk; j++) { k.data[j] = data[j]; k.valid[j] = valid[j]; k.ctype[j] = p_ct[j]; }
+        return k;
+    }
 
     void set_kind(bool is_mark, bool is_anti) {
         B200_REQUIRE(n_build == 0 && !build_final, "b200 join: the join kind must be set before the first build batch");
@@ -730,7 +953,11 @@ class JoinState {
     // ---- runtime join filter ----
     // n_blocks: 32-byte bloom blocks (0 = one per 32 build rows, ~8 bits per key); ranks that will OR their filters together
     // pass the same value.  Also computes the min / max of the (non-NA) build keys.
+    void require_single_key_filter() const {
+        B200_REQUIRE(nk == 1, "b200 join: the runtime join filter is built for single-column join keys only (this state joins on " + std::to_string(nk) + " key columns)");
+    }
     void build_filter(uint64_t n_blocks) {
+        require_single_key_filter();
         B200_REQUIRE(build_final, "b200 join: runtime filter before the build side was finished");
         B200_CUDA(cudaSetDevice(device)); scratch_set_stream(stream);
         bloom_blocks = n_blocks ? n_blocks : (uint64_t)n_build / 32 + 1;
@@ -751,6 +978,7 @@ class JoinState {
         key_min = h[0]; key_max = h[1];
     }
     void runtime_filter(const b200_table* t, int key_col, bool use_minmax, bool use_bloom, uint8_t* keep) {
+        require_single_key_filter();
         B200_REQUIRE(t->device == device, "b200 join: runtime_filter takes a device-resident table on the state's device");
         B200_REQUIRE(key_col >= 0 && key_col < t->n_cols, "b200 join: runtime_filter: bad key column");
         B200_REQUIRE(ctype_size(t->cols[key_col].c_type) == ctype_size(b_ct[0]) && !ctype_is_float(t->cols[key_col].c_type), "b200 join: runtime_filter: key column type differs from the build key");
@@ -820,10 +1048,10 @@ class JoinState {
     }
 
     // Inline-payload build attempt (unique keys expected): true when the Slot32 table is complete, false when a key repeats
-    // (or the schema does not qualify) and the general build has to run.
+    // (or the schema does not qualify: multi-column keys never do) and the general build has to run.
     bool try_inline_build(uint64_t n_slots) {
         const int nf = n_b - 1;
-        bool ok = n_build > 0 && nf <= 2 && !build_outer && !probe_outer && !(getenv("B200_JOIN_INLINE") && getenv("B200_JOIN_INLINE")[0] == '0');
+        bool ok = nk == 1 && n_build > 0 && nf <= 2 && !build_outer && !probe_outer && !(getenv("B200_JOIN_INLINE") && getenv("B200_JOIN_INLINE")[0] == '0');
         for (int c = 0; c < n_b; c++) ok = ok && ctype_size(b_ct[c]) == 8 && !b_has_valid[c];
         if (!ok) return false;
         d_slots32.alloc(n_slots * sizeof(Slot32));
@@ -871,14 +1099,21 @@ class JoinState {
             return;
         }
         d_tkeys.alloc(n_slots * 8);
-        fill_i64_kernel<<<grid_for((int64_t)n_slots), 256, 0, stream>>>(d_tkeys.as<long long>(), n_slots, J_EMPTY);
+        if (nk == 1) fill_i64_kernel<<<grid_for((int64_t)n_slots), 256, 0, stream>>>(d_tkeys.as<long long>(), n_slots, J_EMPTY);
+        else B200_CUDA(cudaMemsetAsync(d_tkeys.p, 0, n_slots * 8, stream));  // every tag TAG_EMPTY
         d_info.alloc(n_slots * sizeof(SlotInfo));
         B200_CUDA(cudaMemsetAsync(d_info.p, 0, n_slots * sizeof(SlotInfo), stream));
         d_row_slot.alloc((size_t)std::max<int64_t>(n_build, 1) * 4);
-        launches++;
+        if (nk == 1) launches++;
         if (n_build > 0) {
-            join_insert_count_kernel<<<grid_for(n_build), 256, 0, stream>>>(bcol[0].buf.p, b_ct[0], b_has_valid[0] ? bvalid[0].buf.as<uint8_t>() : nullptr,
-                                                                           n_build, d_tkeys.as<long long>(), cap, d_info.as<SlotInfo>(), d_row_slot.as<uint32_t>(), na_equal ? 1 : 0);
+            if (nk == 1)
+                join_insert_count_kernel<<<grid_for(n_build), 256, 0, stream>>>(bcol[0].buf.p, b_ct[0], b_has_valid[0] ? bvalid[0].buf.as<uint8_t>() : nullptr,
+                                                                               n_build, d_tkeys.as<long long>(), cap, d_info.as<SlotInfo>(), d_row_slot.as<uint32_t>(), na_equal ? 1 : 0);
+            else
+                with_nk([&](auto k) {
+                    join_insert_count_mk_kernel<decltype(k)::value><<<grid_for(n_build), 256, 0, stream>>>(build_keys(), n_build, d_tkeys.as<unsigned long long>(), cap,
+                                                                                                           d_info.as<SlotInfo>(), d_row_slot.as<uint32_t>(), na_equal ? 1 : 0);
+                });
             d_cnt_multi.alloc(n_slots * 4);
             join_slot_counts_kernel<<<grid_for((int64_t)n_slots), 256, 0, stream>>>(d_info.as<SlotInfo>(), n_slots, d_cnt_multi.as<uint32_t>());
             launches += 2;
@@ -894,15 +1129,18 @@ class JoinState {
             }
             d_cnt_multi.release(); d_fill.release(); d_row_slot.release();
             if (n_multi == 0 && !build_outer && !probe_outer && !mark && !anti && n_b >= 1) {
-                // every key (incl. the NA / marker groups) has exactly one build row: set up the fused probe path
+                // every key (incl. the NA / marker groups) has exactly one build row: set up the fused probe path.  Single key: Slot16.key
+                // is the key and the packed rows hold the non-key columns; multi-key: Slot16.key is the tuple's tag and the packed rows
+                // hold every column (the tuple check reads the keys from there)
                 d_slots16.alloc(n_slots * sizeof(Slot16));
                 join_make_slots16_kernel<<<grid_for((int64_t)n_slots), 256, 0, stream>>>(d_tkeys.as<long long>(), d_info.as<SlotInfo>(), n_slots, d_slots16.as<Slot16>());
-                int nf = n_b - 1;
+                const int c0 = nk == 1 ? 1 : 0;
+                int nf = n_b - c0;
                 d_bpack.alloc((size_t)std::max<int64_t>(n_build * std::max(nf, 1), 1) * 8);
                 if (nf > 0) {
                     PackPayloadArgs pa{};
                     pa.n_build = n_build; pa.n_fields = nf; pa.out = d_bpack.as<unsigned long long>();
-                    for (int c = 1; c < n_b; c++) { pa.src[c - 1] = bcol[c].buf.p; pa.size[c - 1] = ctype_size(b_ct[c]); }
+                    for (int c = c0; c < n_b; c++) { pa.src[c - c0] = bcol[c].buf.p; pa.size[c - c0] = ctype_size(b_ct[c]); }
                     join_pack_payload_kernel<<<grid_for(n_build), 256, 0, stream>>>(pa);
                 }
                 d_cursor.alloc(8);
@@ -944,13 +1182,38 @@ class JoinState {
         for (int k = 0; k < n_out_cols; k++) {
             bool is_b = k < (int)kb.size();
             int src = is_b ? kb[k] : kp[k - kb.size()];
-            out_has_valid[k] = is_b ? (src == 0 ? (valid[0] != nullptr || b_at[0] == ARR_NULLABLE) : (b_has_valid[src] || b_at[src] == ARR_NULLABLE))
+            out_has_valid[k] = is_b ? (src == 0 && nk == 1 ? (valid[0] != nullptr || b_at[0] == ARR_NULLABLE) : (b_has_valid[src] || b_at[src] == ARR_NULLABLE))
                                     : (valid[src] != nullptr || p_at[src] == ARR_NULLABLE);
             out_data[k].ensure((size_t)(n + 32) * ctype_size(is_b ? b_ct[src] : p_ct[src]));  // matches <= probe rows
             if (out_has_valid[k]) { out_vbytes[k].ensure((size_t)n + 32); out_bitmap[k].ensure((size_t)((n + 31) / 32 + 1) * 4); }
         }
         int64_t rows = 0;
-        if (n > 0) {
+        if (n > 0 && nk > 1) {
+            FastProbeMkArgs f{};
+            f.n_probe = n; f.pk = probe_keys(data, valid);
+            for (int j = 0; j < nk; j++) {
+                f.bk_valid[j] = b_has_valid[j] ? bvalid[j].buf.as<uint8_t>() : nullptr;
+                f.bk_bits[j] = ctype_size(b_ct[j]) == 8 ? ~0ull : (1ull << (8 * ctype_size(b_ct[j]))) - 1;
+            }
+            f.slots = d_slots16.as<Slot16>(); f.cap = cap; f.bpack = d_bpack.as<unsigned long long>(); f.n_fields = n_b;
+            f.cursor = d_cursor.as<unsigned long long>(); f.n_b = (int)kb.size(); f.n_p = (int)kp.size(); f.na_equal = na_equal ? 1 : 0;
+            for (int k = 0; k < n_out_cols; k++) {
+                bool is_b = k < (int)kb.size();
+                int src = is_b ? kb[k] : kp[k - kb.size()];
+                if (is_b) {
+                    f.b_field[k] = src; f.b_size[k] = ctype_size(b_ct[src]);
+                    f.b_valid[k] = b_has_valid[src] ? bvalid[src].buf.as<uint8_t>() : nullptr;
+                    f.ob_data[k] = out_data[k].p; f.ob_valid[k] = out_has_valid[k] ? out_vbytes[k].as<uint8_t>() : nullptr;
+                } else {
+                    int j = k - (int)kb.size();
+                    f.p_data[j] = data[src]; f.p_valid[j] = valid[src]; f.p_size[j] = ctype_size(p_ct[src]);
+                    f.op_data[j] = out_data[k].p; f.op_valid[j] = out_has_valid[k] ? out_vbytes[k].as<uint8_t>() : nullptr;
+                }
+            }
+            B200_CUDA(cudaMemsetAsync(d_cursor.p, 0, 8, stream));
+            const int gridp = (int)std::min<int64_t>((int64_t)sms * 8, (n + 1023) / 1024);
+            with_nk([&](auto c) { join_probe_fast_mk_kernel<decltype(c)::value><<<gridp, 256, 0, stream>>>(f); });
+        } else if (n > 0) {
             FastProbeArgs f{};
             f.n_probe = n; f.key_data = data[0]; f.key_ctype = p_ct[0]; f.key_valid = valid[0];
             f.slots = d_slots16.as<Slot16>(); f.cap = cap; f.bpack = d_bpack.as<unsigned long long>(); f.n_fields = std::max(n_b - 1, 1);
@@ -992,6 +1255,8 @@ class JoinState {
                 f.slots = d_slots16.as<Slot16>(); f.bpack = d_bpack.as<unsigned long long>();
                 join_probe_fast_kernel<<<gridp, 256, 0, stream>>>(f);
             }
+        }
+        if (n > 0) {
             launches++; fast_probes++;
             B200_CUDA(cudaGetLastError());
             B200_CUDA(cudaMemcpyAsync(h_cursor, d_cursor.p, 8, cudaMemcpyDeviceToHost, stream));
@@ -1034,9 +1299,16 @@ class JoinState {
         d_pslot.ensure((size_t)(n + 1) * 4); d_pcnt.ensure((size_t)(n + 1) * 4); d_poff.ensure((size_t)(n + 2) * 8);
         if (n > 0) {
             if (mark) { d_mark.ensure((size_t)n + 32); d_mark_valid.ensure((size_t)(n + 7) / 8 + 32); B200_CUDA(cudaMemsetAsync(d_mark_valid.p, 0xff, (size_t)(n + 7) / 8 + 8, stream)); }
-            join_probe_count_kernel<<<grid_for(n), 256, 0, stream>>>(data[0], p_ct[0], valid[0], n, d_tkeys.as<long long>(), cap, d_info.as<SlotInfo>(),
-                                                                     probe_outer ? 1 : 0, d_pslot.as<uint32_t>(), d_pcnt.as<uint32_t>(), na_equal ? 1 : 0,
-                                                                     anti ? 1 : (mark ? 2 : 0), mark ? d_mark.as<uint8_t>() : nullptr);
+            if (nk == 1)
+                join_probe_count_kernel<<<grid_for(n), 256, 0, stream>>>(data[0], p_ct[0], valid[0], n, d_tkeys.as<long long>(), cap, d_info.as<SlotInfo>(),
+                                                                         probe_outer ? 1 : 0, d_pslot.as<uint32_t>(), d_pcnt.as<uint32_t>(), na_equal ? 1 : 0,
+                                                                         anti ? 1 : (mark ? 2 : 0), mark ? d_mark.as<uint8_t>() : nullptr);
+            else
+                with_nk([&](auto c) {
+                    join_probe_count_mk_kernel<decltype(c)::value><<<grid_for(n), 256, 0, stream>>>(
+                        probe_keys(data, valid), build_keys(), n, d_tkeys.as<unsigned long long>(), cap, d_info.as<SlotInfo>(), probe_outer ? 1 : 0,
+                        d_pslot.as<uint32_t>(), d_pcnt.as<uint32_t>(), na_equal ? 1 : 0, anti ? 1 : (mark ? 2 : 0), mark ? d_mark.as<uint8_t>() : nullptr);
+                });
             launches++;
             B200_CUDA(cudaMemsetAsync(d_pcnt.as<uint32_t>() + n, 0, 4, stream));
             n_match = scan.run(d_pcnt.as<uint32_t>(), n + 1, d_poff.as<unsigned long long>(), stream, &launches);
@@ -1217,6 +1489,7 @@ int b200_join_build_filter(void* state, int64_t n_bloom_blocks, void** bloom_wor
 int b200_join_set_key_bounds(void* state, int64_t key_min, int64_t key_max) {
     try {
         B200_REQUIRE(state, "b200 join: null state");
+        ((JoinState*)state)->require_single_key_filter();
         ((JoinState*)state)->key_min = key_min; ((JoinState*)state)->key_max = key_max;
         return 0;
     } catch (const std::exception& e) { b200::set_last_error(e.what()); return -1; }

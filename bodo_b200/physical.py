@@ -241,10 +241,18 @@ class PhysicalAggregate:
         G.delete_groupby_state(self.state)
 
 
-class PhysicalJoin:
-    """Hash join: sink for build batches, ProcessBatch for probe batches (join.h:58-744)."""
+def _key_tuple(keys) -> tuple:
+    """One key (an int or a column name) or a sequence of them, as a tuple."""
+    import numbers
 
-    def __init__(self, build_key: int, probe_key: int, build_names, probe_names, how: str = "inner", **kw):
+    return (keys,) if isinstance(keys, (str, numbers.Integral)) else tuple(keys)
+
+
+class PhysicalJoin:
+    """Hash join: sink for build batches, ProcessBatch for probe batches (join.h:58-744).  `build_key` / `probe_key`: one column
+    index or a sequence of 1..4 (a multi-column equi-join: position j of one side is compared with position j of the other)."""
+
+    def __init__(self, build_key, probe_key, build_names, probe_names, how: str = "inner", **kw):
         build_outer = how in ("right", "outer")   # the build side is the RIGHT table (reference convention)
         probe_outer = how in ("left", "outer")
         if how == "anti":   # LEFT ANTI: probe rows without a partner (physical/join.h:151: no build columns in the output)
@@ -252,7 +260,8 @@ class PhysicalJoin:
         elif how == "mark":
             kw["is_mark_join"] = True
         kw.setdefault("is_na_equal", True)  # pandas merge semantics: NA joins NA (bodo/pandas/physical/join.h:267)
-        self.state = J.init_join_state(-1, (build_key,), (probe_key,), tuple(build_names), tuple(probe_names), build_outer, probe_outer, **kw)
+        bk, pk = tuple(int(k) for k in _key_tuple(build_key)), tuple(int(k) for k in _key_tuple(probe_key))
+        self.state = J.init_join_state(-1, bk, pk, tuple(build_names), tuple(probe_names), build_outer, probe_outer, **kw)
 
     def ConsumeBatch(self, batch: Table, prev: OperatorResult) -> OperatorResult:
         is_last = prev == OperatorResult.FINISHED
@@ -343,11 +352,17 @@ def groupby_agg_parquet(path: str, by, aggs: Sequence[tuple], dropna: bool = Tru
     return out
 
 
-def merge(left, right, left_on: str, right_on: str, how: str = "inner", batch_size: int = STREAMING_BATCH_SIZE, **kw):
+def merge(left, right, left_on, right_on, how: str = "inner", batch_size: int = STREAMING_BATCH_SIZE, **kw):
     """left.merge(right, left_on=..., right_on=..., how=...) through the streaming join (right = build side).
+    `left_on` / `right_on`: a column name or equally long lists of 1..4 names (a multi-column join).
     Output columns: right's columns then left's columns (the reference's build-then-probe order), renamed on clashes."""
+    from ._lib import B200Error
+
+    lon, ron = _key_tuple(left_on), _key_tuple(right_on)
+    if len(lon) != len(ron):
+        raise B200Error(f"merge: left_on and right_on must have the same length (got {len(lon)} and {len(ron)})")
     rcols, lcols = list(right.columns), list(left.columns)
-    op = PhysicalJoin(rcols.index(right_on), lcols.index(left_on), rcols, lcols, how=how, **kw)
+    op = PhysicalJoin(tuple(rcols.index(c) for c in ron), tuple(lcols.index(c) for c in lon), rcols, lcols, how=how, **kw)
     run_pipeline(PhysicalReadPandas(right, batch_size), [], op)
     coll = ResultCollector()
     run_pipeline(PhysicalReadPandas(left, batch_size), [op], coll)

@@ -18,7 +18,8 @@ Here, per rank (one process per GPU, torch.distributed / NCCL for the plumbing):
 
 The calls are collective, as in the reference: every rank calls build / probe the same number of times (ranks that ran out of
 input keep calling with empty batches until the is_last call, bodo/pandas/_pipeline.cpp:453-457).
-Placement is the reference's: (uint32) XXH3_64(key, SEED_HASH_PARTITION) % n_pes.
+Placement is the reference's: (uint32) XXH3_64(key, SEED_HASH_PARTITION) % n_pes, and for 2..4 key columns hash_keys of the
+tuple (the further columns folded in with hash_combine_boost) % n_pes.
 """
 
 from __future__ import annotations
@@ -145,13 +146,15 @@ class DistJoinState:
                                  is_mark_join=is_mark_join, is_anti_join=is_anti_join)
         self.probe_outer = bool(probe_outer)
         # bloom filter + key bounds over the build keys of ALL ranks, applied to probe rows before they are shuffled (the
-        # reference's use_bloom_filter probe path, _join.cpp:3460-3600); B200_JOIN_BLOOM=0 disables it
-        self.use_filter = os.environ.get("B200_JOIN_BLOOM", "1") != "0" and not probe_outer and not is_mark_join and not is_anti_join
+        # reference's use_bloom_filter probe path, _join.cpp:3460-3600); B200_JOIN_BLOOM=0 disables it.  The filter is built for
+        # single-column keys only, so a multi-column join skips it
+        self.build_key = self.local.build_key_inds
+        self.probe_key = self.local.probe_key_inds
+        self.use_filter = (os.environ.get("B200_JOIN_BLOOM", "1") != "0" and not probe_outer and not is_mark_join and not is_anti_join
+                           and len(self.build_key) == 1)
         self.filter_ready = False
         self._build_batches = []
         self.is_broadcast = False
-        self.build_key = self.local.build_key_inds[0]
-        self.probe_key = self.local.probe_key_inds[0]
         self.metrics = {"build_rows_in": 0, "build_rows_local": 0, "probe_rows_in": 0, "probe_rows_local": 0, "broadcast": 0}
 
     # handle / metrics pass-throughs so get_metric / delete work on both kinds of state
@@ -159,27 +162,27 @@ class DistJoinState:
     def handle(self):
         return self.local.handle
 
-    def _keys_first(self, table: Table, key: int) -> Table:
-        order = [key] + [i for i in range(table.n_cols) if i != key]
+    def _keys_first(self, table: Table, keys) -> Table:
+        order = list(keys) + [i for i in range(table.n_cols) if i not in keys]
         return table.select(order), order
 
-    def _shuffle(self, table: Table, key: int) -> Table:
-        """Rows to their owners; returns the rows this rank owns, in the table's original column order."""
+    def _shuffle(self, table: Table, keys) -> Table:
+        """Rows to their owners (hash_keys of the key tuple); returns the rows this rank owns, in the table's original column order."""
         import torch
 
-        kf, order = self._keys_first(to_device(table, self.device), key)
-        part, counts = partition_device(with_schema_validity(kf), 1, self.n_pes)
+        kf, order = self._keys_first(to_device(table, self.device), keys)
+        part, counts = partition_device(with_schema_validity(kf), len(keys), self.n_pes)
         torch.cuda.current_stream().synchronize()
         recv = exchange_table(part, counts, self.group)
         inv = [order.index(i) for i in range(len(order))]
         return recv.select(inv)
 
-    def _owned_only(self, table: Table, key: int) -> Table:
+    def _owned_only(self, table: Table, keys) -> Table:
         """Replicated input against a partitioned other side: keep the rows whose key this rank owns (no exchange)."""
         import torch
 
-        kf, order = self._keys_first(to_device(table, self.device), key)
-        part, counts = partition_device(with_schema_validity(kf), 1, self.n_pes)
+        kf, order = self._keys_first(to_device(table, self.device), keys)
+        part, counts = partition_device(with_schema_validity(kf), len(keys), self.n_pes)
         torch.cuda.current_stream().synchronize()
         lo = sum(counts[: self.rank])
         n = counts[self.rank]
@@ -252,7 +255,7 @@ class DistJoinState:
         partitioned_build = self.build_parallel and not self.is_broadcast
         if partitioned_build and self.probe_parallel:
             if self.filter_ready and table.n_rows:
-                table = J.runtime_join_filter((self,), to_device(table, self.device), ((self.probe_key,),))
+                table = J.runtime_join_filter((self,), to_device(table, self.device), (self.probe_key,))
                 self.metrics["probe_rows_after_filter"] = self.metrics.get("probe_rows_after_filter", 0) + table.n_rows
             table = self._shuffle(table, self.probe_key)
         elif partitioned_build:

@@ -5,7 +5,11 @@ Same verbs and calling protocol as the reference (init_join_state :991-1100, joi
 test loops (bodo/tests/test_streaming/test_join.py) carry over.  The work happens in libbodo_b200.so.
 
 Output column order is the reference's: kept build-table columns first, then kept probe-table columns
-(both in logical input order, the key column included on each side unless dropped through used/kept cols).
+(both in logical input order, the key columns included on each side unless dropped through used/kept cols).
+
+A join takes 1..4 integer / date key columns per side, the same number on both sides; key position j of the build side is
+compared with key position j of the probe side, and both must have the same byte width.  Runtime join filters are built for
+single-column keys only.
 """
 
 from __future__ import annotations
@@ -13,6 +17,8 @@ from __future__ import annotations
 from .. import _lib
 from .._lib import ffi
 from ..table import CTable, Table, table_from_ctable
+
+MAX_KEYS = 4  # equi-join key columns per side (the C state's n_keys limit, as for the groupby and the shuffle)
 
 
 class JoinState:
@@ -24,8 +30,10 @@ class JoinState:
         self.is_anti_join = bool(is_anti_join)
         self.build_key_inds = tuple(int(k) for k in build_key_inds)
         self.probe_key_inds = tuple(int(k) for k in probe_key_inds)
-        if len(self.build_key_inds) != 1 or len(self.probe_key_inds) != 1:
-            raise _lib.B200Error("Streaming Join: exactly one equi-join key per side is supported")
+        nk = len(self.build_key_inds)
+        if not 1 <= nk <= MAX_KEYS or len(self.probe_key_inds) != nk:
+            raise _lib.B200Error(f"Streaming Join: between 1 and {MAX_KEYS} equi-join keys per side, the same number on both sides, are "
+                                 f"supported (got {nk} build and {len(self.probe_key_inds)} probe keys)")
         self.build_colnames = list(build_colnames) if build_colnames is not None else None
         self.probe_colnames = list(probe_colnames) if probe_colnames is not None else None
         self.build_outer = bool(build_outer)
@@ -59,7 +67,7 @@ class JoinState:
 
             self.device = build.device if build.device >= 0 else torch.cuda.current_device()
         h = L.b200_join_state_init(self.operator_id, ffi.new("int8_t[]", bct), ffi.new("int8_t[]", bat), len(bct),
-                                   ffi.NULL, ffi.NULL, 0, 1, int(self.build_outer), int(self.probe_outer), int(self.is_na_equal),
+                                   ffi.NULL, ffi.NULL, 0, len(self.build_key_inds), int(self.build_outer), int(self.probe_outer), int(self.is_na_equal),
                                    self.output_batch_size, self.device, self.expected_build_rows, ffi.cast("void*", self.stream))
         self.handle = _lib.check_ptr(h, "init_join_state")
         if self.is_mark_join or self.is_anti_join:
@@ -175,12 +183,19 @@ def delete_join_state(join_state: JoinState) -> None:
         join_state.handle = None
 
 
+def _require_single_key_filter(st: JoinState, key_idxs=(0,)) -> None:
+    if len(st.build_key_inds) > 1 or len(key_idxs) > 1:
+        raise _lib.B200Error(f"runtime_join_filter: multi-column runtime join filters are not built yet (this join has "
+                             f"{max(len(st.build_key_inds), len(key_idxs))} key columns; single-column keys only)")
+
+
 def build_runtime_filter(join_state, n_bloom_blocks: int = 0):
     """Build the bloom filter + key bounds of a finished build side; returns (bloom words as a device tensor aliasing the
     state's memory, (key_min, key_max)).  Sharded joins OR / min / max these across ranks (dist_join.DistJoinState does)."""
     import torch
 
     st = getattr(join_state, "local", join_state)
+    _require_single_key_filter(st)
     L = _lib.lib()
     ptr = ffi.new("void**")
     nb = ffi.new("int64_t*")
@@ -203,6 +218,8 @@ def runtime_join_filter(join_states, table: Table, join_keys_idxs, process_col_b
     from ..expr import col
     from ..physical import filter_project_table
 
+    for k, js in enumerate(join_states):
+        _require_single_key_filter(getattr(js, "local", js), tuple(join_keys_idxs[k]))
     if table.device < 0:
         raise _lib.B200Error("runtime_join_filter: the table must be device resident")
     L = _lib.lib()

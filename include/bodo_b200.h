@@ -140,10 +140,13 @@ int64_t b200_groupby_get_metric(void* state, int32_t which);
 
 /* ---- streaming hash join (reference: bodo/libs/streaming/_join.cpp) ---- */
 
-/* join_state_init_py_entry (_join.cpp:4087-4136). Inner equi-join on the first n_keys (=1) columns;
- * build_table_outer / probe_table_outer select right/left/full-outer semantics. `is_na_equal` is the
- * HashJoinState option of the same name: 0 (what join_state_init_py_entry constructs: NA keys never match,
- * _join.cpp:3180) or 1 (what bodo/pandas/physical/join.h:267 passes: NA joins NA, pandas merge semantics).
+/* join_state_init_py_entry (_join.cpp:4087-4136). Equi-join on the first n_keys (1..4) columns of each side:
+ * key column j of the build side is compared with key column j of the probe side, on the values widened to
+ * int64; key columns are integer / date / datetime / timedelta / bool typed, and both sides have the same byte
+ * width at every key position. build_table_outer / probe_table_outer select right/left/full-outer semantics.
+ * `is_na_equal` is the HashJoinState option of the same name: 0 (what join_state_init_py_entry constructs:
+ * a row with an NA in ANY key column matches nothing, _join.cpp:3180) or 1 (what bodo/pandas/physical/join.h:267
+ * passes, pandas merge semantics: NA equals NA at the same key position and never equals a value).
  * n_probe_arrs may be 0: the probe schema is then taken from the first probe batch. */
 void* b200_join_state_init(int64_t operator_id, const int8_t* build_arr_c_types,
                            const int8_t* build_arr_array_types, int32_t n_build_arrs,
@@ -176,7 +179,8 @@ void b200_delete_join_state(void* state);
 int b200_join_set_kind(void* state, int32_t is_mark_join, int32_t is_anti_join);
 
 /* Runtime join filter (HashJoinState::RuntimeFilter, _join.h:1060-1095; bloom filter bodo/libs/gpu_bloom_filter.cu:60-201; key
- * min / max _join.cpp:3199-3238), available once the build side is complete.
+ * min / max _join.cpp:3199-3238), available once the build side is complete, for single-column keys only: the three calls return
+ * an error for a state with n_keys > 1.
  * b200_join_build_filter builds a split-block bloom filter over the build keys (n_bloom_blocks 32-byte blocks, 0 = one per 32 build
  * rows) and their min / max; it returns the device address of the filter words (n_blocks * 8 uint32) so that the ranks of a sharded
  * join can OR their filters together in place (all ranks pass the same n_bloom_blocks; b200_join_set_key_bounds installs the
