@@ -972,9 +972,9 @@ __global__ void eval_mk_keys_kernel(const __grid_constant__ EvalMkKeysArgs a) {
 // row cap the direct kernel at ≈85 Grows/s and the key probe halves that again (L2 random-request rate), while
 // 32-bit shared-memory atomics sustain the full HBM stream rate.  So rows travel to the SM that owns their key:
 //
-//   K1 spg_partition_kernel : every CTA counting-sorts TILE-row tiles by owner (= mulhi(hash, n_owners)) in
-//        shared memory, reserves one run per owner with a single global atomic per (tile, owner) and copies
-//        the runs out with coalesced 16-byte stores -> owner buckets of (key, value) rows in HBM.
+//   K1 spg_partition_tma_kernel : every CTA fetches TILE-row tiles with TMA bulk copies, counting-sorts them by owner
+//        (= mulhi(hash, n_owners)) in shared memory, reserves one run per owner with a single global atomic per
+//        (tile, owner) and copies the runs out with coalesced 16-byte stores -> owner buckets of (key, value) rows in HBM.
 //   K2 spg_aggregate_kernel : one CTA per owner streams its bucket into a shared-memory hash table (key CAS,
 //        SUM = two native 32-bit atomics with carry, COUNT = one), then flushes the table into the state's
 //        global table with the ordinary find-or-insert + `red` (each key has one owner: <= n_groups per launch).
@@ -985,8 +985,6 @@ __global__ void eval_mk_keys_kernel(const __grid_constant__ EvalMkKeysArgs a) {
 // inside the same kernels; rows that cannot even be inserted there (global table at its limit) are appended to
 // a retry list in the partial-aggregate wire format and replayed by combine_partials_kernel after the table grew.
 constexpr int SPG_THREADS = 1024;   // K2 (aggregate) threads per CTA
-constexpr int SPG_PTHREADS = 256;   // K1 (partition) threads per CTA
-constexpr int SPG_PCTAS = 4;        // K1 CTAs per SM (more independent CTAs = barrier / load stalls overlap)
 constexpr int SPG_TILE = 2048;
 constexpr int SPG_MAX_OWNERS = 256;
 // K1 reserves one run per owner per tile with a global atomic on the owner's row counter: ~10^7 atomics per launch.  With
@@ -1050,6 +1048,77 @@ __device__ __forceinline__ void spg_direct_apply(const SpgArgs& a, long long key
     }
     if (HAS_SUM && sum) atomicAdd(a.acc_sum + sl, sum);
     if (HAS_CNT && cnt) atomicAdd(a.acc_cnt + sl, cnt);
+}
+
+// ---- steps shared by the K1 / K2 kernels of SPG, SPG-N (spgn.cuh) and SPG-G (spgg.cuh) -------------------------
+// Force-inlined: the kernels were tuned with these steps written out, and `__noinline__` cold paths measured slower.
+
+// K1: exclusive scan of a tile's class histogram hist[0, C) by warp 0 into lbase[0, C); lbase[C] = the tile's rows
+__device__ __forceinline__ void spg_scan_hist(const unsigned int* hist, unsigned int* lbase, int C, int tid) {
+    if (tid < 32) {
+        unsigned int carry = 0;
+        for (int base = 0; base < C; base += 32) {
+            int j = base + tid;
+            unsigned int x = j < C ? hist[j] : 0u, inc = x;
+#pragma unroll
+            for (int d = 1; d < 32; d <<= 1) { unsigned int y = __shfl_up_sync(0xffffffffu, inc, d); if (tid >= d) inc += y; }
+            if (j < C) lbase[j] = carry + inc - x;
+            carry += __shfl_sync(0xffffffffu, inc, 31);
+        }
+        if (tid == 0) lbase[C] = carry;
+    }
+}
+
+// K2 shared tables are two-choice bucketed hash tables + stash: NB two-slot buckets, then SPG_STASH stash slots.
+// The two candidate buckets of the key whose spg_hash is h:
+__device__ __forceinline__ void spg_buckets(uint64_t h, unsigned int NB, unsigned int& b1, unsigned int& b2) {
+    b1 = __umulhi((unsigned int)(h >> 20), NB);
+    b2 = __umulhi(((unsigned int)h ^ (unsigned int)(h >> 44)) * 0x9E3779B1u, NB);  // low word of h remixed: independent of b1's bits 20..51 enough
+    b2 = b2 == b1 ? (b1 + 1 == NB ? 0u : b1 + 1) : b2;
+}
+// the slot holding `key` in bucket b1 (slots c1.x, c1.y) or b2 (c2.x, c2.y), each read with one shared load; -1 = neither
+template <typename P, typename K>
+__device__ __forceinline__ int spg_find_slot(const P& c1, const P& c2, unsigned int b1, unsigned int b2, K key) {
+    return c1.x == key ? (int)(2 * b1) : c1.y == key ? (int)(2 * b1 + 1) : c2.x == key ? (int)(2 * b2) : c2.y == key ? (int)(2 * b2 + 1) : -1;
+}
+// K2 slow path: the key's candidate slot, else a free candidate slot claimed by CAS, else find-or-insert in the stash behind
+// the NS bucket slots; -1 = no room (the caller sends the row the direct way).  Balanced allocation: a new key goes to the
+// EMPTIER of its two buckets (0.9 % of the keys overflow into the stash at 50 % load where first-fit left 2.2 % there —
+// every row of a stash-resident key comes through here), and the four CAS attempts are skipped when both buckets are full
+// (buckets never lose keys), so a stash-resident key costs two loads and one stash probe instead of four failed CAS round
+// trips.  SPG-N's K2n has its own 32-bit copy, see spgn_aggregate_kernel.
+__device__ __forceinline__ int spg_slow_slot(long long* skeys, int NS, unsigned int NB, long long key) {
+    unsigned int b1, b2;
+    spg_buckets(spg_hash(key), NB, b1, b2);
+    const unsigned long long uk = (unsigned long long)key;
+    const ulonglong2 c1 = *reinterpret_cast<const ulonglong2*>(skeys + 2 * b1);
+    const ulonglong2 c2 = *reinterpret_cast<const ulonglong2*>(skeys + 2 * b2);
+    const int f1 = (c1.x == (unsigned long long)EMPTY_KEY) + (c1.y == (unsigned long long)EMPTY_KEY);
+    const int f2 = (c2.x == (unsigned long long)EMPTY_KEY) + (c2.y == (unsigned long long)EMPTY_KEY);
+    int s = spg_find_slot(c1, c2, b1, b2, uk);
+    if (s < 0 && f1 + f2 > 0) {
+        const unsigned int first = f2 > f1 ? b2 : b1, second = f2 > f1 ? b1 : b2;
+        const unsigned int cand[4] = {2 * first, 2 * first + 1, 2 * second, 2 * second + 1};
+#pragma unroll
+        for (int c = 0; c < 4 && s < 0; c++) {
+            unsigned long long old = atomicCAS((unsigned long long*)&skeys[cand[c]], (unsigned long long)EMPTY_KEY, uk);
+            if (old == (unsigned long long)EMPTY_KEY || old == uk) s = (int)cand[c];
+        }
+    }
+    if (s < 0) {
+        unsigned int st = (unsigned int)NS + ((unsigned int)(spg_hash(key) >> 12) & (SPG_STASH - 1));
+        for (int probes = 0; probes < SPG_STASH && s < 0; probes++) {
+            unsigned long long kk = (unsigned long long)skeys[st];
+            if (kk == (unsigned long long)EMPTY_KEY) {
+                unsigned long long old = atomicCAS((unsigned long long*)&skeys[st], (unsigned long long)EMPTY_KEY, uk);
+                if (old == (unsigned long long)EMPTY_KEY) { s = (int)st; break; }
+                kk = old;
+            }
+            if (kk == uk) { s = (int)st; break; }
+            st = st + 1 == (unsigned int)NS + SPG_STASH ? (unsigned int)NS : st + 1;
+        }
+    }
+    return s;
 }
 
 // ---- heavy hitters (skewed keys) ----------------------------------------------------------------------------
@@ -1131,93 +1200,13 @@ __global__ void __launch_bounds__(1024, 1) spg_hot_sample_kernel(const long long
     if (tid == 0) { n_hot[0] = (int)nh; n_hot[1] = (int)nwide; }
 }
 
-// K1 (plain-load fallback, used when the inputs are not 16-byte aligned or B200_SPG_TMA=0): partition rows into owner
-// buckets. grid = persistent (SPG_PCTAS CTAs / SM), tiles are taken grid-stride.
-template <bool HAS_SUM, bool HAS_CNT>
-__global__ void __launch_bounds__(SPG_PTHREADS, SPG_PCTAS) spg_partition_kernel(const __grid_constant__ SpgArgs a) {
-    extern __shared__ __align__(16) unsigned char smem_raw[];
-    longlong2* stage = (longlong2*)smem_raw;                                   // SPG_TILE x 16
-    unsigned long long* gbase = (unsigned long long*)(stage + SPG_TILE);      // SPG_MAX_OWNERS x 8
-    unsigned int* hist = (unsigned int*)(gbase + SPG_MAX_OWNERS);             // SPG_MAX_OWNERS
-    unsigned int* lbase = hist + SPG_MAX_OWNERS;                               // SPG_MAX_OWNERS + 1
-    unsigned char* stage_owner = (unsigned char*)(lbase + SPG_MAX_OWNERS + 4);  // SPG_TILE
-    const int G = a.n_owners, tid = threadIdx.x;
-    constexpr int ROWS = SPG_TILE / SPG_PTHREADS;  // 8 rows per thread per tile, as 4 adjacent pairs
-    constexpr int PAIRS = ROWS / 2;
-    const int64_t n_tiles = (a.n_rows + SPG_TILE - 1) / SPG_TILE;
-    for (int j = tid; j < G; j += SPG_PTHREADS) hist[j] = 0;
-    __syncthreads();
-    for (int64_t t = blockIdx.x; t < n_tiles; t += gridDim.x) {
-        const int64_t r0 = t * SPG_TILE;
-        long long k[ROWS], v[ROWS];
-        int o[ROWS];
-        unsigned int rk[ROWS];
-#pragma unroll
-        for (int j = 0; j < PAIRS; j++) {
-            int64_t i = r0 + ((int64_t)j * SPG_PTHREADS + tid) * 2;
-            if (i + 1 < a.n_rows) {
-                longlong2 t2 = __ldcs(reinterpret_cast<const longlong2*>(a.keys + i));
-                k[2 * j] = t2.x; k[2 * j + 1] = t2.y;
-                if (HAS_SUM) { longlong2 u2 = __ldcs(reinterpret_cast<const longlong2*>(a.vals + i)); v[2 * j] = u2.x; v[2 * j + 1] = u2.y; }
-                else { v[2 * j] = 0; v[2 * j + 1] = 0; }
-                o[2 * j] = 0; o[2 * j + 1] = 0;
-            } else if (i < a.n_rows) {
-                k[2 * j] = a.keys[i]; v[2 * j] = HAS_SUM ? a.vals[i] : 0; o[2 * j] = 0;
-                k[2 * j + 1] = 0; v[2 * j + 1] = 0; o[2 * j + 1] = -1;
-            } else { k[2 * j] = k[2 * j + 1] = 0; v[2 * j] = v[2 * j + 1] = 0; o[2 * j] = o[2 * j + 1] = -1; }
-        }
-#pragma unroll
-        for (int r = 0; r < ROWS; r++) {
-            if (o[r] < 0) continue;
-            if (k[r] == EMPTY_KEY) { spg_direct_apply<HAS_SUM, HAS_CNT>(a, k[r], (unsigned long long)v[r], 1ull); o[r] = -1; continue; }
-            o[r] = (int)spg_owner(spg_hash(k[r]), G);
-            rk[r] = atomicAdd(&hist[o[r]], 1u);
-        }
-        __syncthreads();
-        // reserve one run per owner; exclusive scan of the histogram by warp 0
-        if (tid < G) { unsigned int cnt = hist[tid]; gbase[tid] = cnt ? atomicAdd(&a.bucket_cnt[tid * SPG_CNT_STRIDE], (unsigned long long)cnt) : 0ull; }
-        if (tid < 32) {
-            unsigned int carry = 0;
-            for (int base = 0; base < G; base += 32) {
-                int j = base + tid;
-                unsigned int x = j < G ? hist[j] : 0u, inc = x;
-#pragma unroll
-                for (int d = 1; d < 32; d <<= 1) { unsigned int y = __shfl_up_sync(0xffffffffu, inc, d); if (tid >= d) inc += y; }
-                if (j < G) lbase[j] = carry + inc - x;
-                carry += __shfl_sync(0xffffffffu, inc, 31);
-            }
-            if (tid == 0) lbase[G] = carry;
-        }
-        __syncthreads();
-#pragma unroll
-        for (int r = 0; r < ROWS; r++) {
-            if (o[r] < 0) continue;
-            unsigned int p = lbase[o[r]] + rk[r];
-            stage[p] = make_longlong2(k[r], v[r]);
-            stage_owner[p] = (unsigned char)o[r];
-        }
-        __syncthreads();
-        const unsigned int n_tile = lbase[G];
-        for (unsigned int p = tid; p < n_tile; p += SPG_PTHREADS) {
-            unsigned int ow = stage_owner[p];
-            unsigned long long off = gbase[ow] + (p - lbase[ow]);
-            longlong2 row = stage[p];
-            if (off < (unsigned long long)a.bucket_cap) a.bucket[(size_t)ow * a.bucket_cap + off] = row;
-            else spg_direct_apply<HAS_SUM, HAS_CNT>(a, row.x, (unsigned long long)row.y, 1ull);  // bucket full (skew): direct path
-        }
-        for (int j = tid; j < G; j += SPG_PTHREADS) hist[j] = 0;  // for the next tile (gbase/lbase were consumed above)
-        __syncthreads();
-    }
-}
-
-// K1 (TMA variant): the tile's key and value slabs are fetched with cp.async.bulk (TMA, SASS UBLKCP) into a
-// double-buffered shared-memory staging area while the previous tile is being sorted, completion is signalled on an
-// mbarrier (expect_tx / complete_tx), so no warp ever stalls on an HBM load and no row lives in registers across a
-// barrier.  Everything after the load (hash, shared-memory histogram, run reservation, staging, coalesced 16-byte
-// copy-out) is the algorithm of spg_partition_kernel.
-constexpr int SPG_TTHREADS = 512;  // threads per CTA of the TMA variant (4 rows per thread per tile)
-constexpr int SPG_TBUFS = 1;       // raw tile buffers per CTA (1: next tile streams in during copy-out; 2: full double buffering)
-constexpr int SPG_TCTAS = 3;       // CTAs per SM
+// K1: partition rows into owner buckets.  The tile's key and value slabs are fetched with cp.async.bulk (TMA, SASS UBLKCP)
+// into a shared-memory staging area while the previous tile is being copied out, completion is signalled on an mbarrier
+// (expect_tx / complete_tx), so no warp ever stalls on an HBM load and no row lives in registers across a barrier.  Then:
+// hash, shared-memory histogram, run reservation, staging, coalesced 16-byte copy-out.  grid = persistent (SPG_TCTAS CTAs
+// per SM), tiles are taken grid-stride.
+constexpr int SPG_TTHREADS = 512;  // K1 threads per CTA (4 rows per thread per tile)
+constexpr int SPG_TCTAS = 3;       // K1 CTAs per SM
 
 __device__ __forceinline__ uint32_t smem_u32(const void* p) { return (uint32_t)__cvta_generic_to_shared(p); }
 __device__ __forceinline__ void mbar_init(uint64_t* bar, uint32_t count) {
@@ -1240,11 +1229,11 @@ __device__ __forceinline__ void tma_load_1d(void* smem_dst, const void* gsrc, ui
 template <bool HAS_SUM, bool HAS_CNT, bool HOT = false>
 __global__ void __launch_bounds__(SPG_TTHREADS, SPG_TCTAS) spg_partition_tma_kernel(const __grid_constant__ SpgArgs a) {
     extern __shared__ __align__(128) unsigned char smem_tma_raw[];  // own name: the other kernels declare smem_raw with 16-byte alignment
-    long long* raw_k = (long long*)smem_tma_raw;                                   // [NB][SPG_TILE] keys
-    long long* raw_v = raw_k + SPG_TBUFS * SPG_TILE;                           // [NB][SPG_TILE] values
-    longlong2* stage = (longlong2*)(raw_v + SPG_TBUFS * SPG_TILE);             // SPG_TILE x 16
+    long long* raw_k = (long long*)smem_tma_raw;                               // [SPG_TILE] keys
+    long long* raw_v = raw_k + SPG_TILE;                                       // [SPG_TILE] values
+    longlong2* stage = (longlong2*)(raw_v + SPG_TILE);                         // SPG_TILE x 16
     unsigned long long* gbase = (unsigned long long*)(stage + SPG_TILE);      // SPG_MAX_OWNERS x 8
-    uint64_t* mbar = (uint64_t*)(gbase + SPG_MAX_OWNERS);                      // 2 mbarriers
+    uint64_t* mbar = (uint64_t*)(gbase + SPG_MAX_OWNERS);                      // 2 mbarriers (one used)
     unsigned int* hist = (unsigned int*)(mbar + 2);                            // SPG_MAX_OWNERS
     unsigned int* lbase = hist + SPG_MAX_OWNERS;                               // SPG_MAX_OWNERS + 1
     unsigned char* stage_owner = (unsigned char*)(lbase + SPG_MAX_OWNERS + 4);  // SPG_TILE
@@ -1261,41 +1250,35 @@ __global__ void __launch_bounds__(SPG_TTHREADS, SPG_TCTAS) spg_partition_tma_ker
     const int64_t n_tiles = (a.n_rows + SPG_TILE - 1) / SPG_TILE;
     if (tid == 0) {
         mbar_init(&mbar[0], 1);
-        mbar_init(&mbar[1], 1);
+        mbar_init(&mbar[1], 1);  // unused (one raw tile buffer); initialised anyway, which keeps K1's SASS the tuned kernel's
         asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
     }
     for (int j = tid; j < G; j += SPG_TTHREADS) hist[j] = 0;
     __syncthreads();
     // full tiles come in through TMA; a trailing partial tile is loaded with ordinary loads
-    auto issue = [&](int64_t t, int b) {
+    auto issue = [&](int64_t t) {
         const int64_t r0 = t * SPG_TILE;
-        if (r0 + SPG_TILE <= a.n_rows) {
-            if (tid == 0) {
-                mbar_expect_tx(&mbar[b], (HAS_SUM ? 2u : 1u) * SPG_TILE * 8u);
-                tma_load_1d(raw_k + b * SPG_TILE, a.keys + r0, SPG_TILE * 8u, &mbar[b]);
-                if (HAS_SUM) tma_load_1d(raw_v + b * SPG_TILE, a.vals + r0, SPG_TILE * 8u, &mbar[b]);
-            }
+        if (r0 + SPG_TILE <= a.n_rows && tid == 0) {
+            mbar_expect_tx(&mbar[0], (HAS_SUM ? 2u : 1u) * SPG_TILE * 8u);
+            tma_load_1d(raw_k, a.keys + r0, SPG_TILE * 8u, &mbar[0]);
+            if (HAS_SUM) tma_load_1d(raw_v, a.vals + r0, SPG_TILE * 8u, &mbar[0]);
         }
     };
-    uint32_t phase[2] = {0, 0};
+    uint32_t phase = 0;
     int64_t t = blockIdx.x;
-    int b = 0;
-    if (t < n_tiles) issue(t, 0);
-    for (; t < n_tiles; t += gridDim.x, b ^= (SPG_TBUFS - 1)) {
+    if (t < n_tiles) issue(t);
+    for (; t < n_tiles; t += gridDim.x) {
         const int64_t r0 = t * SPG_TILE;
         const int64_t tn = t + gridDim.x;
-        if (SPG_TBUFS == 2 && tn < n_tiles) issue(tn, b ^ 1);  // prefetch the next tile of this CTA while this one is sorted
         const bool full = r0 + SPG_TILE <= a.n_rows;
-        long long* kb = raw_k + b * SPG_TILE;
-        long long* vb = raw_v + b * SPG_TILE;
         if (full) {
-            while (!mbar_try_wait(&mbar[b], phase[b])) {}
-            phase[b] ^= 1;
+            while (!mbar_try_wait(&mbar[0], phase)) {}
+            phase ^= 1;
         } else {
             for (int j = tid; j < SPG_TILE; j += SPG_TTHREADS) {
                 int64_t i = r0 + j;
-                kb[j] = i < a.n_rows ? a.keys[i] : 0;
-                vb[j] = (HAS_SUM && i < a.n_rows) ? a.vals[i] : 0;
+                raw_k[j] = i < a.n_rows ? a.keys[i] : 0;
+                raw_v[j] = (HAS_SUM && i < a.n_rows) ? a.vals[i] : 0;
             }
             __syncthreads();
         }
@@ -1306,8 +1289,8 @@ __global__ void __launch_bounds__(SPG_TTHREADS, SPG_TCTAS) spg_partition_tma_ker
             const int j = r * SPG_TTHREADS + tid;
             o[r] = -1;
             if (r0 + j >= a.n_rows) continue;
-            const long long k = kb[j];
-            if (k == EMPTY_KEY) { spg_direct_apply<HAS_SUM, HAS_CNT>(a, k, HAS_SUM ? (unsigned long long)vb[j] : 0ull, 1ull); continue; }
+            const long long k = raw_k[j];
+            if (k == EMPTY_KEY) { spg_direct_apply<HAS_SUM, HAS_CNT>(a, k, HAS_SUM ? (unsigned long long)raw_v[j] : 0ull, 1ull); continue; }
             const uint64_t h = spg_hash(k);
             if (hot_on) {  // heavy hitter: aggregate here, the row never reaches an owner bucket
                 const unsigned int hb = spg_hot_bucket(h);
@@ -1315,7 +1298,7 @@ __global__ void __launch_bounds__(SPG_TTHREADS, SPG_TCTAS) spg_partition_tma_ker
                 const int hs = hk2.x == (unsigned long long)k ? (int)(2 * hb) : hk2.y == (unsigned long long)k ? (int)(2 * hb + 1) : -1;
                 if (hs >= 0) {
                     if (HAS_SUM) {
-                        const unsigned long long v = (unsigned long long)vb[j];
+                        const unsigned long long v = (unsigned long long)raw_v[j];
                         const unsigned int lo = (unsigned int)v;
                         unsigned int hi = (unsigned int)(v >> 32);
                         const unsigned int old = atomicAdd(&hlo[hs], lo);
@@ -1334,31 +1317,20 @@ __global__ void __launch_bounds__(SPG_TTHREADS, SPG_TCTAS) spg_partition_tma_ker
         // after the staging pass, which needs the local prefix sums but not the global run start
         unsigned long long my_gbase = 0;
         if (tid >= SPG_TTHREADS - G) { int ow = tid - (SPG_TTHREADS - G); unsigned int cnt = hist[ow]; if (cnt) my_gbase = atomicAdd(&a.bucket_cnt[ow * SPG_CNT_STRIDE], (unsigned long long)cnt); }
-        if (tid < 32) {
-            unsigned int carry = 0;
-            for (int base = 0; base < G; base += 32) {
-                int j = base + tid;
-                unsigned int x = j < G ? hist[j] : 0u, inc = x;
-#pragma unroll
-                for (int d = 1; d < 32; d <<= 1) { unsigned int y = __shfl_up_sync(0xffffffffu, inc, d); if (tid >= d) inc += y; }
-                if (j < G) lbase[j] = carry + inc - x;
-                carry += __shfl_sync(0xffffffffu, inc, 31);
-            }
-            if (tid == 0) lbase[G] = carry;
-        }
+        spg_scan_hist(hist, lbase, G, tid);
         __syncthreads();
 #pragma unroll
         for (int r = 0; r < ROWS; r++) {
             if (o[r] < 0) continue;
             const int j = r * SPG_TTHREADS + tid;
             unsigned int p = lbase[o[r]] + rk[r];
-            stage[p] = make_longlong2(kb[j], HAS_SUM ? vb[j] : 0);
+            stage[p] = make_longlong2(raw_k[j], HAS_SUM ? raw_v[j] : 0);
             stage_owner[p] = (unsigned char)o[r];
         }
         // publish run start minus local start, so the copy-out computes its destination with one add
         if (tid >= SPG_TTHREADS - G) { int ow = tid - (SPG_TTHREADS - G); gbase[ow] = my_gbase - lbase[ow]; }
-        __syncthreads();  // raw buffer b is free from here on
-        if (SPG_TBUFS == 1 && tn < n_tiles) issue(tn, 0);  // single buffer: the next tile streams in during the copy-out
+        __syncthreads();  // the raw tile is free from here on
+        if (tn < n_tiles) issue(tn);  // the next tile streams in during the copy-out
         const unsigned int n_tile = lbase[G];
         for (unsigned int p = tid; p < n_tile; p += SPG_TTHREADS) {
             unsigned int ow = stage_owner[p];
@@ -1400,12 +1372,6 @@ __global__ void __launch_bounds__(SPG_THREADS, 1) spg_aggregate_kernel(const __g
     const unsigned int NB = (unsigned int)NS / 2;
     const unsigned int NP = (unsigned int)a.n_pass, GP = (unsigned int)gridDim.x * NP;
 
-    auto buckets = [&](long long key, unsigned int& b1, unsigned int& b2) {
-        const uint64_t h = spg_hash(key);
-        b1 = __umulhi((unsigned int)(h >> 20), NB);
-        b2 = __umulhi(((unsigned int)h ^ (unsigned int)(h >> 44)) * 0x9E3779B1u, NB);  // low word of h remixed: independent of b1's bits 20..51 enough
-        b2 = b2 == b1 ? (b1 + 1 == NB ? 0u : b1 + 1) : b2;
-    };
     auto add = [&](int s, long long key, long long val) {
         if (HAS_SUM) {
             unsigned int lo = (unsigned int)(unsigned long long)val, hi = (unsigned int)((unsigned long long)val >> 32);
@@ -1415,42 +1381,9 @@ __global__ void __launch_bounds__(SPG_THREADS, 1) spg_aggregate_kernel(const __g
         }
         if (HAS_CNT) atomicAdd(&scnt[s], 1u);
     };
-    // slow path: claim a free candidate slot, else find-or-insert in the stash, else the direct global path.
-    // Balanced allocation: a new key goes to the EMPTIER of its two buckets (0.9 % of the keys overflow into the stash
-    // at 50 % load where first-fit left 2.2 % there — every row of a stash-resident key comes through here), and the four
-    // CAS attempts are skipped when both buckets are full (buckets never lose keys), so a stash-resident key costs two
-    // loads and one stash probe instead of four failed CAS round trips.
+    // slow path (spg_slow_slot), else the direct global path
     auto slow_upsert = [&](long long key, long long val) {
-        unsigned int b1, b2;
-        buckets(key, b1, b2);
-        const unsigned long long uk = (unsigned long long)key;
-        const ulonglong2 c1 = *reinterpret_cast<const ulonglong2*>(skeys + 2 * b1);
-        const ulonglong2 c2 = *reinterpret_cast<const ulonglong2*>(skeys + 2 * b2);
-        const int f1 = (c1.x == (unsigned long long)EMPTY_KEY) + (c1.y == (unsigned long long)EMPTY_KEY);
-        const int f2 = (c2.x == (unsigned long long)EMPTY_KEY) + (c2.y == (unsigned long long)EMPTY_KEY);
-        int s = c1.x == uk ? (int)(2 * b1) : c1.y == uk ? (int)(2 * b1 + 1) : c2.x == uk ? (int)(2 * b2) : c2.y == uk ? (int)(2 * b2 + 1) : -1;
-        if (s < 0 && f1 + f2 > 0) {
-            const unsigned int first = f2 > f1 ? b2 : b1, second = f2 > f1 ? b1 : b2;
-            const unsigned int cand[4] = {2 * first, 2 * first + 1, 2 * second, 2 * second + 1};
-#pragma unroll
-            for (int c = 0; c < 4 && s < 0; c++) {
-                unsigned long long old = atomicCAS((unsigned long long*)&skeys[cand[c]], (unsigned long long)EMPTY_KEY, uk);
-                if (old == (unsigned long long)EMPTY_KEY || old == uk) s = (int)cand[c];
-            }
-        }
-        if (s < 0) {
-            unsigned int st = (unsigned int)NS + ((unsigned int)(spg_hash(key) >> 12) & (SPG_STASH - 1));
-            for (int probes = 0; probes < SPG_STASH && s < 0; probes++) {
-                unsigned long long kk = (unsigned long long)skeys[st];
-                if (kk == (unsigned long long)EMPTY_KEY) {
-                    unsigned long long old = atomicCAS((unsigned long long*)&skeys[st], (unsigned long long)EMPTY_KEY, uk);
-                    if (old == (unsigned long long)EMPTY_KEY) { s = (int)st; break; }
-                    kk = old;
-                }
-                if (kk == uk) { s = (int)st; break; }
-                st = st + 1 == (unsigned int)NS + SPG_STASH ? (unsigned int)NS : st + 1;
-            }
-        }
+        const int s = spg_slow_slot(skeys, NS, NB, key);
         if (s < 0) { spg_direct_apply<HAS_SUM, HAS_CNT>(a, key, (unsigned long long)val, 1ull); return; }
         add(s, key, val);
     };
@@ -1472,11 +1405,10 @@ __global__ void __launch_bounds__(SPG_THREADS, 1) spg_aggregate_kernel(const __g
 #pragma unroll
         for (int u = 0; u < U; u++) {  // hot lookups: branch-free
             unsigned int b1, b2;
-            buckets(row[u].x, b1, b2);
+            spg_buckets(spg_hash(row[u].x), NB, b1, b2);
             const ulonglong2 k1 = *reinterpret_cast<const ulonglong2*>(skeys + 2 * b1);
             const ulonglong2 k2 = *reinterpret_cast<const ulonglong2*>(skeys + 2 * b2);
-            const unsigned long long uk = (unsigned long long)row[u].x;
-            sl[u] = k1.x == uk ? (int)(2 * b1) : k1.y == uk ? (int)(2 * b1 + 1) : k2.x == uk ? (int)(2 * b2) : k2.y == uk ? (int)(2 * b2 + 1) : -1;
+            sl[u] = spg_find_slot(k1, k2, b1, b2, (unsigned long long)row[u].x);
             if (!FULL && row[u].x == EMPTY_KEY) sl[u] = -2;  // padding lane
             // multi-pass: owner = mulhi(hash_hi, G) = mulhi(hash_hi, G * NP) / NP; this pass keeps sub-range `pass` only
             if (NP > 1 && __umulhi((unsigned int)(spg_hash(row[u].x) >> 32), GP) - (unsigned int)me * NP != pass) sl[u] = -2;
@@ -1904,6 +1836,13 @@ class GroupbyState {
         cap = new_cap;
         rebuilds++;
     }
+    // grow the table (at least doubling it) until n_groups + pending groups fit under its group limit of cap / 2
+    void grow_to_hold(int64_t pending) {
+        uint64_t nc = cap;
+        while (nc < 2ull * (uint64_t)(n_groups + pending)) nc <<= 1;
+        if (nc == cap) nc <<= 1;
+        grow(nc);
+    }
 
     // ---- multi-key table management ----
     void alloc_mk(uint64_t c, DevBuf& tags, DevBuf* mk, DevBuf& mask) {
@@ -1973,10 +1912,7 @@ class GroupbyState {
         while (h_counters[1] > 0) {
             int64_t nf = h_counters[1];
             fail_rows += nf;
-            uint64_t nc = cap;
-            while (nc < 2ull * (uint64_t)(n_groups + nf)) nc <<= 1;
-            if (nc == cap) nc <<= 1;
-            grow(nc);
+            grow_to_hold(nf);
             // the fail list becomes the index list of the replay; it cannot fail again (room for nf new groups)
             DevBuf replay_list;
             replay_list.alloc((size_t)nf * 4);
@@ -1998,6 +1934,22 @@ class GroupbyState {
     int64_t spg_launches = 0, spg_retry_rows = 0, lc_launches = 0;
     int64_t expected_groups_hint = 0;
 
+    // Calls f(std::bool_constant<HAS_SUM>, std::bool_constant<HAS_CNT>) for the accumulators of the int64 fast path: sum and
+    // count, sum only or count only (sum_j / cnt_j < 0: not asked for).  These are the three instantiations of its kernels.
+    template <typename F>
+    static void with_sum_cnt(int sum_j, int cnt_j, F&& f) {
+        if (sum_j >= 0 && cnt_j >= 0) f(std::true_type{}, std::true_type{});
+        else if (sum_j >= 0) f(std::true_type{}, std::false_type{});
+        else f(std::false_type{}, std::true_type{});
+    }
+    // ... and f for each of the three
+    template <typename F>
+    static void for_each_sum_cnt(F&& f) {
+        f(std::true_type{}, std::true_type{});
+        f(std::true_type{}, std::false_type{});
+        f(std::false_type{}, std::true_type{});
+    }
+
     bool spg_probe() {
         if (spg_state >= 0) return spg_state == 1;
         spg_state = 0;
@@ -2008,31 +1960,29 @@ class GroupbyState {
         if (sms > SPG_MAX_OWNERS - 1 || max_smem < 64 * 1024) return false;
         spg_ns = ((int)(((size_t)max_smem - 64) / 16) - SPG_STASH) & ~1;
         spg_smem = (size_t)(spg_ns + SPG_STASH) * 16 + 16;
-        const void* fns[3] = {(const void*)spg_aggregate_kernel<true, true>, (const void*)spg_aggregate_kernel<true, false>,
-                              (const void*)spg_aggregate_kernel<false, true>};
-        for (auto f : fns)
-            if (cudaFuncSetAttribute(f, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)spg_smem) != cudaSuccess) { cudaGetLastError(); return false; }
-        const void* pf[3] = {(const void*)spg_partition_kernel<true, true>, (const void*)spg_partition_kernel<true, false>,
-                             (const void*)spg_partition_kernel<false, true>};
-        for (auto f : pf)
-            if (cudaFuncSetAttribute(f, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)spg_part_smem()) != cudaSuccess) { cudaGetLastError(); return false; }
-        const void* tf[3] = {(const void*)spg_partition_tma_kernel<true, true>, (const void*)spg_partition_tma_kernel<true, false>,
-                             (const void*)spg_partition_tma_kernel<false, true>};
-        for (auto f : tf)
-            if (cudaFuncSetAttribute(f, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)spg_tma_smem()) != cudaSuccess) { cudaGetLastError(); return false; }
-        const void* hf[3] = {(const void*)spg_partition_tma_kernel<true, true, true>, (const void*)spg_partition_tma_kernel<true, false, true>,
-                             (const void*)spg_partition_tma_kernel<false, true, true>};
-        for (auto f : hf)
-            if (cudaFuncSetAttribute(f, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)spg_tma_smem(true)) != cudaSuccess) { cudaGetLastError(); return false; }
-        { const char* e2 = getenv("B200_SPG_TMA"); spg_use_tma = !(e2 && e2[0] == '0'); }
+        // opt a kernel in to `bytes` of dynamic shared memory; false (error cleared) when the device refuses
+        auto smem_ok = [](const void* f, size_t bytes) {
+            if (cudaFuncSetAttribute(f, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bytes) == cudaSuccess) return true;
+            cudaGetLastError();
+            return false;
+        };
+        bool ok = true;
+        for_each_sum_cnt([&](auto S, auto C) {
+            constexpr bool HS = decltype(S)::value, HC = decltype(C)::value;
+            ok = ok && smem_ok((const void*)spg_aggregate_kernel<HS, HC>, spg_smem) &&
+                 smem_ok((const void*)spg_partition_tma_kernel<HS, HC>, spg_tma_smem()) &&
+                 smem_ok((const void*)spg_partition_tma_kernel<HS, HC, true>, spg_tma_smem(true));
+        });
+        if (!ok) return false;
         {   // SPG-N (spgn.cuh): narrow bucket rows
             spgn_ns = ((int)(((size_t)max_smem - 256) / 12) - SPG_STASH) & ~1;  // (K2n also has a few static shared words)
             spgn_smem = (size_t)(spgn_ns + SPG_STASH) * 12 + 16;
-            const void* nk1[3] = {(const void*)spgn_partition_kernel<true, true>, (const void*)spgn_partition_kernel<true, false>, (const void*)spgn_partition_kernel<false, true>};
-            const void* nk2[3] = {(const void*)spgn_aggregate_kernel<true, true>, (const void*)spgn_aggregate_kernel<true, false>, (const void*)spgn_aggregate_kernel<false, true>};
             spgn_enabled = true;
-            for (auto f : nk1) if (cudaFuncSetAttribute(f, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)spgn_part_smem()) != cudaSuccess) { cudaGetLastError(); spgn_enabled = false; }
-            for (auto f : nk2) if (cudaFuncSetAttribute(f, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)spgn_smem) != cudaSuccess) { cudaGetLastError(); spgn_enabled = false; }
+            for_each_sum_cnt([&](auto S, auto C) {
+                constexpr bool HS = decltype(S)::value, HC = decltype(C)::value;
+                if (!smem_ok((const void*)spgn_partition_kernel<HS, HC>, spgn_part_smem())) spgn_enabled = false;
+                if (!smem_ok((const void*)spgn_aggregate_kernel<HS, HC>, spgn_smem)) spgn_enabled = false;
+            });
             const char* e8 = getenv("B200_SPG_NARROW");
             if (e8 && e8[0] == '0') spgn_enabled = false;
         }
@@ -2041,7 +1991,7 @@ class GroupbyState {
             const void* gp[6] = {(const void*)spgg_partition_kernel<8, 8>, (const void*)spgg_partition_kernel<8, 4>, (const void*)spgg_partition_kernel<8, 0>,
                                  (const void*)spgg_partition_kernel<4, 8>, (const void*)spgg_partition_kernel<4, 4>, (const void*)spgg_partition_kernel<4, 0>};
             for (auto f : gp)
-                if (cudaFuncSetAttribute(f, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)GEN_K1_SMEM) != cudaSuccess) { cudaGetLastError(); spgg_enabled = false; }
+                if (!smem_ok(f, GEN_K1_SMEM)) spgg_enabled = false;
             for (int v = 0; v < 4; v++) {  // v = mm + 2 * nn
                 const int sb = 16 + ((v & 1) ? 16 : 0) + ((v & 2) ? 4 : 0);
                 spgg_ns[v] = ((int)(((size_t)max_smem - 64) / sb) - SPG_STASH) & ~1;
@@ -2052,17 +2002,17 @@ class GroupbyState {
                                  (const void*)spgg_aggregate_kernel<false, false, true>, (const void*)spgg_aggregate_kernel<true, false, true>,
                                  (const void*)spgg_aggregate_kernel<false, true, true>, (const void*)spgg_aggregate_kernel<true, true, true>};
             for (int q = 0; q < 8; q++)  // q = sum + 2 * mm + 4 * nn
-                if (cudaFuncSetAttribute(ga[q], cudaFuncAttributeMaxDynamicSharedMemorySize, (int)spgg_smem[q >> 1]) != cudaSuccess) { cudaGetLastError(); spgg_enabled = false; }
+                if (!smem_ok(ga[q], spgg_smem[q >> 1])) spgg_enabled = false;
             const char* e7 = getenv("B200_SPG_GEN");
             if (e7 && e7[0] == '0') spgg_enabled = false;
         }
-        if (cudaFuncSetAttribute((const void*)spg_hot_sample_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)SPG_HOT_SAMPLE_SMEM) != cudaSuccess) { cudaGetLastError(); return false; }
+        if (!smem_ok((const void*)spg_hot_sample_kernel, SPG_HOT_SAMPLE_SMEM)) return false;
         { const char* e4 = getenv("B200_SPG_HOT"); spg_hot_enabled = !(e4 && e4[0] == '0'); }
         d_hot.alloc((size_t)SPG_HOT_SLOTS * 8 + 16);
-        const void* lf[3] = {(const void*)groupby_lowcard_kernel<true, true, LC_SLOTS_BIG, 2>, (const void*)groupby_lowcard_kernel<true, false, LC_SLOTS_BIG, 2>,
-                             (const void*)groupby_lowcard_kernel<false, true, LC_SLOTS_BIG, 2>};
-        for (auto f : lf)
-            if (cudaFuncSetAttribute(f, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)((size_t)LC_SLOTS_BIG * 20 + 64)) != cudaSuccess) { cudaGetLastError(); return false; }
+        for_each_sum_cnt([&](auto S, auto C) {
+            ok = ok && smem_ok((const void*)groupby_lowcard_kernel<decltype(S)::value, decltype(C)::value, LC_SLOTS_BIG, 2>, (size_t)LC_SLOTS_BIG * 20 + 64);
+        });
+        if (!ok) return false;
         { const char* e3 = getenv("B200_LC"); lc_enabled = !(e3 && e3[0] == '0'); }
         spg_owners = sms;  // one owner (bucket + shared table) per SM
         d_bucket_cnt.alloc((size_t)std::max(2 * spg_owners, GEN_CLS) * SPG_CNT_STRIDE * 8);  // SPG-G: one counter per class of K1g
@@ -2070,7 +2020,7 @@ class GroupbyState {
         return true;
     }
 
-    bool spg_use_tma = true, lc_enabled = true, lowcard_small = false;
+    bool lc_enabled = true, lowcard_small = false;
     // SPG-N: narrow bucket rows (spgn.cuh)
     int spgn_ns = 0;
     size_t spgn_smem = 0;
@@ -2093,8 +2043,7 @@ class GroupbyState {
         int64_t p = (est + spg_group_capacity() - 1) / spg_group_capacity();
         return p <= 1 ? 1 : (p <= SPG_MAX_PASSES ? (int)p : 0);
     }
-    static size_t spg_tma_smem(bool hot = false) { return (size_t)SPG_TILE * (16 * SPG_TBUFS + 16 + 1) + SPG_MAX_OWNERS * 8 + 16 + (2 * SPG_MAX_OWNERS + 4) * 4 + (hot ? SPG_HOT_SLOTS * 20 : 0) + 256; }
-    static size_t spg_part_smem() { return (size_t)SPG_TILE * 17 + SPG_MAX_OWNERS * 8 + (2 * SPG_MAX_OWNERS + 4) * 4 + 64; }
+    static size_t spg_tma_smem(bool hot = false) { return (size_t)SPG_TILE * (16 + 16 + 1) + SPG_MAX_OWNERS * 8 + 16 + (2 * SPG_MAX_OWNERS + 4) * 4 + (hot ? SPG_HOT_SLOTS * 20 : 0) + 256; }
     bool lc_pick(int64_t est) { lowcard_small = est <= LC_SLOTS_SMALL / 4; return lc_enabled && est <= LC_SLOTS_BIG / 4; }
     // groups the shared-memory tables of all owners are expected to hold together (two-choice buckets work well up to ~70 %)
     int64_t spg_group_capacity() const { return (int64_t)spg_owners * (spg_ns * 7 / 10); }
@@ -2117,14 +2066,11 @@ class GroupbyState {
             spg_retry_rows += nr;
             B200_CUDA(cudaStreamSynchronize(stream));  // the other in-flight launch uses the table we are about to replace
             read_counters();
-            uint64_t nc = cap;
             int64_t pending = h_counters[1] + h_counters[6];
             // the snapshot this call was made on may be stale: the other slot's spg_finish already grew the table and merged
             // BOTH retry lists (their live counters are 0 then) — nothing left to do, and no second grow
             if (pending == 0) break;
-            while (nc < 2ull * (uint64_t)(n_groups + pending + (int64_t)spg_owners * spg_ns)) nc <<= 1;
-            if (nc == cap) nc <<= 1;
-            grow(nc);
+            grow_to_hold(pending + (int64_t)spg_owners * spg_ns);
             for (int sl = 0; sl < 2; sl++) {
                 int64_t cnt = h_counters[1 + 5 * sl];
                 if (cnt == 0) continue;
@@ -2155,10 +2101,11 @@ class GroupbyState {
         }
         double tspg0 = now();
         struct Acc2 { double& t; double t0; ~Acc2() { t += now() - t0; } } acc2{t_spg, tspg0};
+        B200_REQUIRE(((uintptr_t)keys & 15) == 0 && ((uintptr_t)vals & 15) == 0,
+                     "internal: the SM-partitioned groupby takes 16-byte aligned columns (K1 fetches tiles with TMA bulk copies)");
         read_counters();  // exact group count before the first launch
         n_groups_bound = n_groups;
-        const bool tma_all = spg_use_tma && (((uintptr_t)keys & 15) == 0) && (vals == nullptr || ((uintptr_t)vals & 15) == 0);
-        if (!lowcard && tma_all && !spg_hot_sampled) {
+        if (!lowcard && !spg_hot_sampled) {
             // once per state: count a sample of this call's keys (heavy hitters) and test the sampled rows against the narrow-row
             // format; the host reads back both verdicts
             int* d_nhot = (int*)(d_hot.as<long long>() + SPG_HOT_SLOTS);
@@ -2171,7 +2118,7 @@ class GroupbyState {
             launches++;
         }
         // narrow bucket rows are half the bytes: twice the rows per launch for the same scratch, half the per-launch flushes
-        const bool narrow_call = spgn_enabled && !lowcard && tma_all && spg_n_hot == 0 && spg_sample_wide == 0;
+        const bool narrow_call = spgn_enabled && !lowcard && spg_n_hot == 0 && spg_sample_wide == 0;
         const int64_t launch_rows = narrow_call ? 2 * SPG_LAUNCH_ROWS : SPG_LAUNCH_ROWS;
         int64_t li = 0;
         for (int64_t r0 = 0; r0 < n; r0 += launch_rows, li++) {
@@ -2203,25 +2150,19 @@ class GroupbyState {
                 const bool small = lowcard_small;
                 int gl = (int)std::min<int64_t>((int64_t)sms * (small ? 3 : 2), (rows + LC_THREADS * 2 - 1) / (LC_THREADS * 2));
                 size_t lsm = (size_t)(small ? LC_SLOTS_SMALL : LC_SLOTS_BIG) * 20 + 64;
-                if (small) {
-                    if (sum_j >= 0 && cnt_j >= 0) groupby_lowcard_kernel<true, true, LC_SLOTS_SMALL, 3><<<gl, LC_THREADS, lsm, stream>>>(a);
-                    else if (sum_j >= 0) groupby_lowcard_kernel<true, false, LC_SLOTS_SMALL, 3><<<gl, LC_THREADS, lsm, stream>>>(a);
-                    else groupby_lowcard_kernel<false, true, LC_SLOTS_SMALL, 3><<<gl, LC_THREADS, lsm, stream>>>(a);
-                } else {
-                    if (sum_j >= 0 && cnt_j >= 0) groupby_lowcard_kernel<true, true, LC_SLOTS_BIG, 2><<<gl, LC_THREADS, lsm, stream>>>(a);
-                    else if (sum_j >= 0) groupby_lowcard_kernel<true, false, LC_SLOTS_BIG, 2><<<gl, LC_THREADS, lsm, stream>>>(a);
-                    else groupby_lowcard_kernel<false, true, LC_SLOTS_BIG, 2><<<gl, LC_THREADS, lsm, stream>>>(a);
-                }
+                with_sum_cnt(sum_j, cnt_j, [&](auto S, auto C) {
+                    constexpr bool HS = decltype(S)::value, HC = decltype(C)::value;
+                    if (small) groupby_lowcard_kernel<HS, HC, LC_SLOTS_SMALL, 3><<<gl, LC_THREADS, lsm, stream>>>(a);
+                    else groupby_lowcard_kernel<HS, HC, LC_SLOTS_BIG, 2><<<gl, LC_THREADS, lsm, stream>>>(a);
+                });
                 lc_launches++;
             } else {
-                int g1 = (int)std::min<int64_t>((int64_t)sms * SPG_PCTAS, (rows + SPG_TILE - 1) / SPG_TILE);
-                const bool tma = spg_use_tma && (((uintptr_t)a.keys & 15) == 0) && (a.vals == nullptr || ((uintptr_t)a.vals & 15) == 0);
-                int g2 = (int)std::min<int64_t>((int64_t)sms * SPG_TCTAS, (rows + SPG_TILE - 1) / SPG_TILE);
-                const bool hot = tma && spg_hot_enabled && spg_n_hot > 0;
+                int g1 = (int)std::min<int64_t>((int64_t)sms * SPG_TCTAS, (rows + SPG_TILE - 1) / SPG_TILE);
+                const bool hot = spg_hot_enabled && spg_n_hot > 0;
                 if (hot) { a.hot_tab = d_hot.as<long long>(); a.n_hot = (const int*)(d_hot.as<long long>() + SPG_HOT_SLOTS); }
                 const size_t tsm = spg_tma_smem(hot);
                 // SPG-N: the sample found only rows that fit (int32 key, int32 value), and the rows that did not so far are rare
-                const bool narrow = spgn_enabled && tma && !hot && spg_sample_wide == 0 && spgn_wide_rows * 64 <= rows_consumed;
+                const bool narrow = spgn_enabled && !hot && spg_sample_wide == 0 && spgn_wide_rows * 64 <= rows_consumed;
                 if (narrow) {
                     a.ns = spgn_ns;
                     // first flush into an empty table: per-CTA ticket reservation, but only with >= 25 % head room under the group
@@ -2233,26 +2174,20 @@ class GroupbyState {
                     a.n_pass = (int)std::min<int64_t>(SPG_MAX_PASSES, std::max<int64_t>(1, (est_n + spgn_group_capacity() - 1) / spgn_group_capacity()));
                     a.bucket_cap = bucket_cap & ~1ll;
                     const size_t nsm = spgn_part_smem();
-                    const int g2 = (int)std::min<int64_t>((int64_t)sms * SPGN_CTAS, (rows + SPGN_TILE - 1) / SPGN_TILE);
-                    if (sum_j >= 0 && cnt_j >= 0) { spgn_partition_kernel<true, true><<<g2, SPG_TTHREADS, nsm, stream>>>(a); spgn_aggregate_kernel<true, true><<<spg_owners, SPG_THREADS, spgn_smem, stream>>>(a); }
-                    else if (sum_j >= 0) { spgn_partition_kernel<true, false><<<g2, SPG_TTHREADS, nsm, stream>>>(a); spgn_aggregate_kernel<true, false><<<spg_owners, SPG_THREADS, spgn_smem, stream>>>(a); }
-                    else { spgn_partition_kernel<false, true><<<g2, SPG_TTHREADS, nsm, stream>>>(a); spgn_aggregate_kernel<false, true><<<spg_owners, SPG_THREADS, spgn_smem, stream>>>(a); }
+                    const int gn = (int)std::min<int64_t>((int64_t)sms * SPGN_CTAS, (rows + SPGN_TILE - 1) / SPGN_TILE);
+                    with_sum_cnt(sum_j, cnt_j, [&](auto S, auto C) {
+                        constexpr bool HS = decltype(S)::value, HC = decltype(C)::value;
+                        spgn_partition_kernel<HS, HC><<<gn, SPG_TTHREADS, nsm, stream>>>(a);
+                        spgn_aggregate_kernel<HS, HC><<<spg_owners, SPG_THREADS, spgn_smem, stream>>>(a);
+                    });
                     spgn_launches++;
-                } else if (sum_j >= 0 && cnt_j >= 0) {
-                    if (hot) spg_partition_tma_kernel<true, true, true><<<g2, SPG_TTHREADS, tsm, stream>>>(a);
-                    else if (tma) spg_partition_tma_kernel<true, true><<<g2, SPG_TTHREADS, tsm, stream>>>(a);
-                    else spg_partition_kernel<true, true><<<g1, SPG_PTHREADS, spg_part_smem(), stream>>>(a);
-                    spg_aggregate_kernel<true, true><<<spg_owners, SPG_THREADS, spg_smem, stream>>>(a);
-                } else if (sum_j >= 0) {
-                    if (hot) spg_partition_tma_kernel<true, false, true><<<g2, SPG_TTHREADS, tsm, stream>>>(a);
-                    else if (tma) spg_partition_tma_kernel<true, false><<<g2, SPG_TTHREADS, tsm, stream>>>(a);
-                    else spg_partition_kernel<true, false><<<g1, SPG_PTHREADS, spg_part_smem(), stream>>>(a);
-                    spg_aggregate_kernel<true, false><<<spg_owners, SPG_THREADS, spg_smem, stream>>>(a);
                 } else {
-                    if (hot) spg_partition_tma_kernel<false, true, true><<<g2, SPG_TTHREADS, tsm, stream>>>(a);
-                    else if (tma) spg_partition_tma_kernel<false, true><<<g2, SPG_TTHREADS, tsm, stream>>>(a);
-                    else spg_partition_kernel<false, true><<<g1, SPG_PTHREADS, spg_part_smem(), stream>>>(a);
-                    spg_aggregate_kernel<false, true><<<spg_owners, SPG_THREADS, spg_smem, stream>>>(a);
+                    with_sum_cnt(sum_j, cnt_j, [&](auto S, auto C) {
+                        constexpr bool HS = decltype(S)::value, HC = decltype(C)::value;
+                        if (hot) spg_partition_tma_kernel<HS, HC, true><<<g1, SPG_TTHREADS, tsm, stream>>>(a);
+                        else spg_partition_tma_kernel<HS, HC><<<g1, SPG_TTHREADS, tsm, stream>>>(a);
+                        spg_aggregate_kernel<HS, HC><<<spg_owners, SPG_THREADS, spg_smem, stream>>>(a);
+                    });
                 }
             }
             B200_CUDA(cudaGetLastError());
@@ -2371,10 +2306,7 @@ class GroupbyState {
             while (h_counters[1] > 0) {  // partials that found the global table at its limit: grow, replay them
                 const int64_t nr = h_counters[1];
                 spg_retry_rows += nr;
-                uint64_t nc = cap;
-                while (nc < 2ull * (uint64_t)(n_groups + nr)) nc <<= 1;
-                if (nc == cap) nc <<= 1;
-                grow(nc);
+                grow_to_hold(nr);
                 d_retry2[1].ensure(device, (size_t)nr * GEN_RETRY_WORDS * 8);
                 B200_CUDA(cudaMemcpyAsync(d_retry2[1].p, d_retry2[0].p, (size_t)nr * GEN_RETRY_WORDS * 8, cudaMemcpyDeviceToDevice, stream));
                 B200_CUDA(cudaMemsetAsync((char*)d_counters.p + 8, 0, 8, stream));
@@ -2478,12 +2410,10 @@ class GroupbyState {
                 const long long* v = vcol >= 0 ? (const long long*)data[vcol] : nullptr;
                 unsigned long long* as = sum_j >= 0 ? d_a0[sum_j].as<unsigned long long>() : nullptr;
                 unsigned long long* ac = cnt_j >= 0 ? d_a0[cnt_j].as<unsigned long long>() : nullptr;
-                if (sum_j >= 0 && cnt_j >= 0)
-                    groupby_consume_i64_sumcount_kernel<true, true><<<g, 256, 0, stream>>>(k, v, rows, d_keys.as<long long>(), cap, as, ac, ctr, limit, d_fail.as<uint32_t>());
-                else if (sum_j >= 0)
-                    groupby_consume_i64_sumcount_kernel<true, false><<<g, 256, 0, stream>>>(k, v, rows, d_keys.as<long long>(), cap, as, ac, ctr, limit, d_fail.as<uint32_t>());
-                else
-                    groupby_consume_i64_sumcount_kernel<false, true><<<g, 256, 0, stream>>>(k, v, rows, d_keys.as<long long>(), cap, as, ac, ctr, limit, d_fail.as<uint32_t>());
+                with_sum_cnt(sum_j, cnt_j, [&](auto S, auto C) {
+                    groupby_consume_i64_sumcount_kernel<decltype(S)::value, decltype(C)::value>
+                        <<<g, 256, 0, stream>>>(k, v, rows, d_keys.as<long long>(), cap, as, ac, ctr, limit, d_fail.as<uint32_t>());
+                });
             } else {
                 ConsumeArgs a = generic_args(data, valid, index_list, rows);
                 groupby_consume_kernel<<<grid_for(rows), 256, 0, stream>>>(a);
@@ -2747,10 +2677,7 @@ class GroupbyState {
                 // received rows that found the table at its group limit: grow, merge them from the slab (still intact), evaluate again
                 int64_t nf = h_counters[1];
                 fail_rows += nf;
-                uint64_t nc = cap;
-                while (nc < 2ull * (uint64_t)(n_groups + nf)) nc <<= 1;
-                if (nc == cap) nc <<= 1;
-                grow(nc);
+                grow_to_hold(nf);
                 DevBuf replay_list;
                 replay_list.alloc((size_t)nf * 4);
                 B200_CUDA(cudaMemcpyAsync(replay_list.p, d_fail.p, (size_t)nf * 4, cudaMemcpyDeviceToDevice, stream));

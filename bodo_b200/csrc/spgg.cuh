@@ -187,18 +187,7 @@ __global__ void __launch_bounds__(SPG_TTHREADS, SPG_TCTAS) spgg_partition_kernel
         __syncthreads();
         unsigned long long my_gbase = 0;
         if (tid >= SPG_TTHREADS - C) { int c = tid - (SPG_TTHREADS - C); unsigned int cnt = hist[c]; if (cnt) my_gbase = atomicAdd(&a.bucket_cnt[c * SPG_CNT_STRIDE], (unsigned long long)cnt); }
-        if (tid < 32) {
-            unsigned int carry = 0;
-            for (int base = 0; base < C; base += 32) {
-                int j = base + tid;
-                unsigned int x = j < C ? hist[j] : 0u, inc = x;
-#pragma unroll
-                for (int d = 1; d < 32; d <<= 1) { unsigned int y = __shfl_up_sync(0xffffffffu, inc, d); if (tid >= d) inc += y; }
-                if (j < C) lbase[j] = carry + inc - x;
-                carry += __shfl_sync(0xffffffffu, inc, 31);
-            }
-            if (tid == 0) lbase[C] = carry;
-        }
+        spg_scan_hist(hist, lbase, C, tid);
         __syncthreads();
 #pragma unroll
         for (int r = 0; r < ROWS; r++) {
@@ -253,12 +242,6 @@ __global__ void __launch_bounds__(SPG_THREADS, 1) spgg_aggregate_kernel(const __
     const bool VO = g.n_vo != a.n_owners;  // bucket me * NP + pass holds exactly this pass's rows
     const bool CHK = NP > 1 && !VO;        // else every row of the owner's bucket is tested against the pass
 
-    auto buckets = [&](long long key, unsigned int& b1, unsigned int& b2) {
-        const uint64_t h = spg_hash(key);
-        b1 = __umulhi((unsigned int)(h >> 20), NB);
-        b2 = __umulhi(((unsigned int)h ^ (unsigned int)(h >> 44)) * 0x9E3779B1u, NB);
-        b2 = b2 == b1 ? (b1 + 1 == NB ? 0u : b1 + 1) : b2;
-    };
     auto add = [&](int s, long long key, long long val) {
         if (HAS_SUM) {
             unsigned int lo = (unsigned int)(unsigned long long)val, hi = (unsigned int)((unsigned long long)val >> 32);
@@ -272,42 +255,8 @@ __global__ void __launch_bounds__(SPG_THREADS, 1) spgg_aggregate_kernel(const __
             if (val > smax[s]) atomicMax(&smax[s], val);
         }
     };
-    // slow path: claim a free candidate slot, else find-or-insert in the stash; -1 = no room (the row goes the direct way)
-    auto slow_slot = [&](long long key) -> int {
-        unsigned int b1, b2;
-        buckets(key, b1, b2);
-        const unsigned long long uk = (unsigned long long)key;
-        const ulonglong2 c1 = *reinterpret_cast<const ulonglong2*>(skeys + 2 * b1);
-        const ulonglong2 c2 = *reinterpret_cast<const ulonglong2*>(skeys + 2 * b2);
-        const int f1 = (c1.x == (unsigned long long)EMPTY_KEY) + (c1.y == (unsigned long long)EMPTY_KEY);
-        const int f2 = (c2.x == (unsigned long long)EMPTY_KEY) + (c2.y == (unsigned long long)EMPTY_KEY);
-        int s = c1.x == uk ? (int)(2 * b1) : c1.y == uk ? (int)(2 * b1 + 1) : c2.x == uk ? (int)(2 * b2) : c2.y == uk ? (int)(2 * b2 + 1) : -1;
-        if (s < 0 && f1 + f2 > 0) {
-            const unsigned int first = f2 > f1 ? b2 : b1, second = f2 > f1 ? b1 : b2;
-            const unsigned int cand[4] = {2 * first, 2 * first + 1, 2 * second, 2 * second + 1};
-#pragma unroll
-            for (int c = 0; c < 4 && s < 0; c++) {
-                unsigned long long old = atomicCAS((unsigned long long*)&skeys[cand[c]], (unsigned long long)EMPTY_KEY, uk);
-                if (old == (unsigned long long)EMPTY_KEY || old == uk) s = (int)cand[c];
-            }
-        }
-        if (s < 0) {
-            unsigned int st = (unsigned int)NS + ((unsigned int)(spg_hash(key) >> 12) & (SPG_STASH - 1));
-            for (int probes = 0; probes < SPG_STASH && s < 0; probes++) {
-                unsigned long long kk = (unsigned long long)skeys[st];
-                if (kk == (unsigned long long)EMPTY_KEY) {
-                    unsigned long long old = atomicCAS((unsigned long long*)&skeys[st], (unsigned long long)EMPTY_KEY, uk);
-                    if (old == (unsigned long long)EMPTY_KEY) { s = (int)st; break; }
-                    kk = old;
-                }
-                if (kk == uk) { s = (int)st; break; }
-                st = st + 1 == (unsigned int)NS + SPG_STASH ? (unsigned int)NS : st + 1;
-            }
-        }
-        return s;
-    };
     auto slow_upsert = [&](long long key, long long val) {
-        const int s = slow_slot(key);
+        const int s = spg_slow_slot(skeys, NS, NB, key);
         if (s < 0) { gen_direct_apply(g, key, (unsigned long long)val, 1ull, 0ull, val, val); return; }
         add(s, key, val);
     };
@@ -330,11 +279,10 @@ __global__ void __launch_bounds__(SPG_THREADS, 1) spgg_aggregate_kernel(const __
 #pragma unroll
         for (int u = 0; u < U; u++) {
             unsigned int b1, b2;
-            buckets(row[u].x, b1, b2);
+            spg_buckets(spg_hash(row[u].x), NB, b1, b2);
             const ulonglong2 k1 = *reinterpret_cast<const ulonglong2*>(skeys + 2 * b1);
             const ulonglong2 k2 = *reinterpret_cast<const ulonglong2*>(skeys + 2 * b2);
-            const unsigned long long uk = (unsigned long long)row[u].x;
-            sl[u] = k1.x == uk ? (int)(2 * b1) : k1.y == uk ? (int)(2 * b1 + 1) : k2.x == uk ? (int)(2 * b2) : k2.y == uk ? (int)(2 * b2 + 1) : -1;
+            sl[u] = spg_find_slot(k1, k2, b1, b2, (unsigned long long)row[u].x);
             if (!FULL && row[u].x == EMPTY_KEY) sl[u] = -2;
             if (CHK && __umulhi((unsigned int)(spg_hash(row[u].x) >> 32), GP) - (unsigned int)me * NP != pass) sl[u] = -2;
         }
@@ -369,7 +317,7 @@ __global__ void __launch_bounds__(SPG_THREADS, 1) spgg_aggregate_kernel(const __
         for (unsigned long long p = tid; p < n_null; p += SPG_THREADS) {
             const long long key = __ldcs(nsrc + p);
             if (NP > 1 && __umulhi((unsigned int)(spg_hash(key) >> 32), GP) - (unsigned int)me * NP != pass) continue;
-            const int s = slow_slot(key);  // looks the four candidates up first
+            const int s = spg_slow_slot(skeys, NS, NB, key);  // looks the four candidates up first
             if (s < 0) gen_direct_apply(g, key, 0ull, 0ull, 1ull, 0, 0);
             else if (HAS_NN) atomicAdd(&snull[s], 1u);
         }

@@ -103,18 +103,7 @@ __global__ void __launch_bounds__(SPG_TTHREADS, SPGN_CTAS) spgn_partition_kernel
         unsigned long long my_gbase = 0;
         unsigned int my_cnt = 0;
         if (tid >= SPG_TTHREADS - G) { int ow = tid - (SPG_TTHREADS - G); my_cnt = hist[ow]; if (my_cnt) my_gbase = atomicAdd(&a.bucket_cnt[ow * SPG_CNT_STRIDE], (unsigned long long)my_cnt); }
-        if (tid < 32) {
-            unsigned int carry = 0;
-            for (int base = 0; base < G; base += 32) {
-                int j = base + tid;
-                unsigned int x = j < G ? hist[j] : 0u, inc = x;
-#pragma unroll
-                for (int d = 1; d < 32; d <<= 1) { unsigned int y = __shfl_up_sync(0xffffffffu, inc, d); if (tid >= d) inc += y; }
-                if (j < G) lbase[j] = carry + inc - x;
-                carry += __shfl_sync(0xffffffffu, inc, 31);
-            }
-            if (tid == 0) lbase[G] = carry;
-        }
+        spg_scan_hist(hist, lbase, G, tid);
         __syncthreads();
 #pragma unroll
         for (int r = 0; r < ROWS; r++) {
@@ -170,11 +159,6 @@ __global__ void __launch_bounds__(SPG_THREADS, 1) spgn_aggregate_kernel(const __
     const unsigned int NB = (unsigned int)NS / 2;
     const unsigned int NP = (unsigned int)a.n_pass, GP = (unsigned int)gridDim.x * NP;
 
-    auto buckets = [&](uint64_t h, unsigned int& b1, unsigned int& b2) {
-        b1 = __umulhi((unsigned int)(h >> 20), NB);
-        b2 = __umulhi(((unsigned int)h ^ (unsigned int)(h >> 44)) * 0x9E3779B1u, NB);
-        b2 = b2 == b1 ? (b1 + 1 == NB ? 0u : b1 + 1) : b2;
-    };
     auto add = [&](int s, int key, int val) {
         if (HAS_SUM) {
             const unsigned int lo = (unsigned int)val;
@@ -185,13 +169,15 @@ __global__ void __launch_bounds__(SPG_THREADS, 1) spgn_aggregate_kernel(const __
         }
         if (HAS_CNT) atomicAdd(&scnt[s], 1u);
     };
+    // spg_slow_slot for 32-bit keys, written out: calling a shared 32-bit instantiation of it changed the register allocation
+    // of the count-only kernel (53 -> 55 registers)
     auto slow_upsert = [&](int key, int val) {
         unsigned int b1, b2;
-        buckets(spg_hash((long long)key), b1, b2);
+        spg_buckets(spg_hash((long long)key), NB, b1, b2);
         const int2 c1 = *reinterpret_cast<const int2*>(skeys + 2 * b1);
         const int2 c2 = *reinterpret_cast<const int2*>(skeys + 2 * b2);
         const int f1 = (c1.x == SPGN_EMPTY) + (c1.y == SPGN_EMPTY), f2 = (c2.x == SPGN_EMPTY) + (c2.y == SPGN_EMPTY);
-        int s = c1.x == key ? (int)(2 * b1) : c1.y == key ? (int)(2 * b1 + 1) : c2.x == key ? (int)(2 * b2) : c2.y == key ? (int)(2 * b2 + 1) : -1;
+        int s = spg_find_slot(c1, c2, b1, b2, key);
         if (s < 0 && f1 + f2 > 0) {
             const unsigned int first = f2 > f1 ? b2 : b1, second = f2 > f1 ? b1 : b2;
             const unsigned int cand[4] = {2 * first, 2 * first + 1, 2 * second, 2 * second + 1};
@@ -243,11 +229,11 @@ __global__ void __launch_bounds__(SPG_THREADS, 1) spgn_aggregate_kernel(const __
         for (int u = 0; u < U; u++) {
             const uint64_t h = spg_hash((long long)row[u].x);
             unsigned int b1, b2;
-            buckets(h, b1, b2);
+            spg_buckets(h, NB, b1, b2);
             const int2 k1 = *reinterpret_cast<const int2*>(skeys + 2 * b1);
             const int2 k2 = *reinterpret_cast<const int2*>(skeys + 2 * b2);
             const int key = row[u].x;
-            sl[u] = k1.x == key ? (int)(2 * b1) : k1.y == key ? (int)(2 * b1 + 1) : k2.x == key ? (int)(2 * b2) : k2.y == key ? (int)(2 * b2 + 1) : -1;
+            sl[u] = spg_find_slot(k1, k2, b1, b2, key);
             if (!FULL && key == SPGN_EMPTY) sl[u] = -2;  // padding lane (INT32_MIN never reaches a bucket)
             if (NP > 1 && __umulhi((unsigned int)(h >> 32), GP) - (unsigned int)me * NP != pass) sl[u] = -2;
         }
